@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the fused view-synthesis loss (BASELINE.json metric: reproj-loss fwd+bwd frames/s).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--workload NAME]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--workload NAME] [--dump-outputs DIR]
 
 Own arm: a "step" is one md2_view_synthesis_loss call (generate_images_pred + compute_losses +
 the adjoint to the 4 disparities and the poses) over one synthetic batch of 12 frames per GPU,
@@ -279,7 +279,16 @@ class PublicStep:
             v.grad = None
         losses = self.fn(self.plan, self.ins, dict(self.leaves))
         losses["loss"].backward()
-        return losses["loss"].detach()
+        self.losses = {k: v.detach() for k, v in losses.items()}
+        return self.losses["loss"]
+
+    def results(self):
+        """What a caller of the public call receives from the last step: the losses dict and the gradients of the
+        disparity and pose leaves, by file-name-safe names."""
+        out = {k.replace("/", "_"): v for k, v in self.losses.items()}
+        for k, v in self.leaves.items():
+            out["grad_" + "_".join(str(x) for x in k)] = v.grad
+        return out
 
     def capture(self):
         cur = torch.cuda.current_stream()
@@ -301,6 +310,21 @@ class PublicStep:
             self.graph.replay()
         else:
             self.loss = self.run()
+
+
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(arrays, out_dir):
+    """Writes every array as <out_dir>/<name>.npy in float32, so that two builds can be compared output for output."""
+    import numpy as np
+    host = {name: t.detach().float().cpu().numpy() for name, t in arrays.items()}
+    total = sum(a.nbytes for a in host.values())
+    if total > DUMP_LIMIT_BYTES:
+        raise RuntimeError("--dump-outputs: %d bytes exceed the %d-byte limit" % (total, DUMP_LIMIT_BYTES))
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in host.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 def quantise_u8(x):
@@ -369,6 +393,9 @@ def run_own(args, wl):
 
     # ---- value: the public call (noise drawn inside, autograd wrapper and backward() included), inputs resident
     # in HBM, one CUDA graph per rotating batch
+    # the public call draws its tie-break noise from the default generator: seeded, every run with the same arguments
+    # computes on the same inputs
+    torch.manual_seed(0)
     pub = [PublicStep(plan, b, dev) for b in host]
     if not args.no_graph:
         for p in pub:
@@ -376,6 +403,8 @@ def run_own(args, wl):
     ms_total, clocks = timed(lambda i: pub[i % nrot].step(), args.steps, max(args.warmup, 3), sample_clocks=True)
     value = world * BATCH * args.steps / (ms_total * 1e-3)
     loss_val = float(pub[(args.steps - 1) % nrot].loss.item())
+    if args.dump_outputs and rank == 0:
+        dump_outputs(pub[(args.steps - 1) % nrot].results(), args.dump_outputs)
 
     # ---- the raw C-ABI call with pre-drawn noise tensors (round 1's headline; kept as an extra key): what the
     # library itself costs without the 4 torch.randn draws and the autograd wrapper
@@ -704,7 +733,14 @@ def main():
     ap.add_argument("--num-layers", type=int, default=18, choices=[18, 50], help="--mode train: ResNet depth")
     ap.add_argument("--no-train", action="store_true", help="skip the training-step sub-record of the default mode")
     ap.add_argument("--bucket-mb", type=int, default=25, help="DDP bucket_cap_mb of the training-step record")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="fused loss path only (--impl own --mode loss): write the losses and gradients of the last "
+                         "timed step of the public call as DIR/<name>.npy (float32)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.mode == "train" or args.impl == "reference"):
+        ap.error("--dump-outputs applies to the fused loss path (--impl own --mode loss)")
     if args.mode == "train":
         run_train(args, args.workload)
     elif args.impl == "reference":

@@ -1,19 +1,28 @@
-"""The drop-in boundary against the reference's own definitions (CPU; needs /root/reference, which exists in
-the build container only - skipped elsewhere): same public names in layers.py, same constructor / call
-signatures, the two Trainer methods the mixin overrides, and LossPlan.from_opt on the real option parser."""
+"""The drop-in boundary against the reference's own definitions (CPU): same public names in layers.py, same
+constructor / call signatures, the two Trainer methods the mixin overrides, and LossPlan.from_opt on the options the
+reference's parser produces for each flag set - as stored in tests/golden/reference_interface.json, which
+tests/golden/make_reference_interface.py records from the reference.  The run_epoch test drives the reference's own
+Trainer and runs where MD2_REFERENCE_DIR names a checkout of the reference."""
+import copy
 import inspect
+import json
 import os
 import sys
 import types
 
 import pytest
 
-REF = "/root/reference"
-pytestmark = pytest.mark.skipif(not os.path.isdir(REF), reason="/root/reference is not present on this box")
+from helpers import GOLDEN_DIR
+
+REF = os.environ.get("MD2_REFERENCE_DIR", "")
+with open(os.path.join(GOLDEN_DIR, "reference_interface.json")) as f:
+    GOLD = json.load(f)
 
 
 @pytest.fixture(scope="module")
 def ref():
+    if not os.path.isdir(REF):
+        pytest.skip("MD2_REFERENCE_DIR does not name a checkout of the reference")
     for name, attrs in (("tensorboardX", {"SummaryWriter": object}), ("IPython", {"embed": lambda *a, **k: None}),
                         ("skimage", {}), ("skimage.transform", {})):
         m = types.ModuleType(name)
@@ -36,10 +45,15 @@ def _params(fn):
     return [p.name for p in inspect.signature(fn).parameters.values()]
 
 
-def test_layers_exports_every_public_name_of_the_reference(ref):
+def _reference_options(flags):
+    """The namespace the reference's MonodepthOptions().parse() returns for `train.py <flags>` (the fields the loss
+    path reads)."""
+    return types.SimpleNamespace(**copy.deepcopy(GOLD["options"][" ".join(flags)]))
+
+
+def test_layers_exports_every_public_name_of_the_reference():
     from monodepth2_b200 import layers as L
-    ref_public = [n for n, v in vars(ref.layers).items()
-                  if not n.startswith("_") and getattr(v, "__module__", None) == ref.layers.__name__]
+    ref_public = GOLD["layers_public"]
     assert ref_public, "nothing found in the reference's layers.py"
     missing = [n for n in ref_public if not hasattr(L, n)]
     assert missing == []
@@ -47,25 +61,31 @@ def test_layers_exports_every_public_name_of_the_reference(ref):
 
 
 @pytest.mark.parametrize("name", ["BackprojectDepth", "Project3D", "SSIM", "ConvBlock", "Conv3x3"])
-def test_module_signatures_match(ref, name):
+def test_module_signatures_match(name):
     from monodepth2_b200 import layers as L
-    a, b = getattr(ref.layers, name), getattr(L, name)
-    assert _params(a.__init__) == _params(b.__init__), name
-    assert _params(a.forward) == _params(b.forward), name
+    a, b = GOLD["modules"][name], getattr(L, name)
+    assert a["__init__"] == _params(b.__init__), name
+    assert a["forward"] == _params(b.forward), name
 
 
 @pytest.mark.parametrize("name", ["disp_to_depth", "transformation_from_parameters", "get_translation_matrix",
                                   "rot_from_axisangle", "get_smooth_loss", "upsample", "compute_depth_errors"])
-def test_function_signatures_match(ref, name):
+def test_function_signatures_match(name):
     from monodepth2_b200 import layers as L
-    assert _params(getattr(ref.layers, name)) == _params(getattr(L, name)), name
+    assert GOLD["functions"][name] == _params(getattr(L, name)), name
 
 
-def test_mixin_overrides_exactly_the_two_hot_path_methods(ref):
+def test_mixin_overrides_exactly_the_two_hot_path_methods():
     from monodepth2_b200.fused_loss import FusedLossMixin
-    T = ref.trainer.Trainer
     for m in ("generate_images_pred", "compute_losses"):
-        assert _params(getattr(T, m)) == _params(getattr(FusedLossMixin, m)), m
+        assert GOLD["trainer_methods"][m] == _params(getattr(FusedLossMixin, m)), m
+
+    class T:                  # stand-in for the reference's Trainer: the methods the mixin leaves to it
+        def process_batch(self, inputs):
+            pass
+
+        def predict_poses(self, inputs, features):
+            pass
 
     class FusedTrainer(FusedLossMixin, T):
         pass
@@ -75,7 +95,7 @@ def test_mixin_overrides_exactly_the_two_hot_path_methods(ref):
     assert FusedTrainer.predict_poses is T.predict_poses
     # the two consumers of the side outputs are wrapped (they materialise what they read, then delegate)
     for m in ("log", "compute_depth_losses"):
-        assert _params(getattr(T, m)) == _params(getattr(FusedLossMixin, m)), m
+        assert GOLD["trainer_methods"][m] == _params(getattr(FusedLossMixin, m)), m
     overridden = [n for n, v in vars(FusedLossMixin).items() if callable(v) and not n.startswith("_")]
     assert sorted(overridden) == ["compute_depth_losses", "compute_losses", "generate_images_pred", "log"]
 
@@ -204,13 +224,12 @@ def test_reference_run_epoch_drives_the_mixin_through_logging_and_val(ref, monke
                                    ["--no_ssim"], ["--v1_multiscale"], ["--pose_model_type", "posecnn"],
                                    ["--disable_automasking", "--predictive_mask"],
                                    ["--height", "320", "--width", "1024"], ["--frame_ids", "0", "--use_stereo"]])
-def test_plan_from_the_reference_option_parser(ref, flags, monkeypatch):
+def test_plan_from_the_reference_option_parser(flags):
     from monodepth2_b200 import _capi
     from monodepth2_b200.fused_loss import LossPlan
     if not os.path.exists(_capi.LIB_PATH):
         pytest.skip("libmd2loss.so not built")
-    monkeypatch.setattr(sys, "argv", ["train.py"] + flags)
-    opt = ref.Options().parse()
+    opt = _reference_options(flags)
     if opt.use_stereo:
         opt.frame_ids.append("s")                                    # trainer.py:51-52
     plan = LossPlan.from_opt(opt)
@@ -224,12 +243,11 @@ def test_plan_from_the_reference_option_parser(ref, flags, monkeypatch):
                                                                           opt.disparity_smoothness)
 
 
-def test_predictive_mask_without_disable_automasking_raises_like_the_reference(ref, monkeypatch):
+def test_predictive_mask_without_disable_automasking_raises_like_the_reference():
     from monodepth2_b200 import _capi
     from monodepth2_b200.fused_loss import LossPlan
     if not os.path.exists(_capi.LIB_PATH):
         pytest.skip("libmd2loss.so not built")
-    monkeypatch.setattr(sys, "argv", ["train.py", "--predictive_mask"])
-    opt = ref.Options().parse()
+    opt = _reference_options(["--predictive_mask"])
     with pytest.raises(RuntimeError):                                # trainer.py:90-92 asserts the same
         LossPlan.from_opt(opt)

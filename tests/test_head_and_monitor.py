@@ -2,45 +2,30 @@
 8f-4  the disparity head of DepthDecoder, sigmoid(Conv3x3(C -> 1)(x))  (networks/depth_decoder.py:60-63,
       layers.py:119-136) as one fused forward pass + a two-pass backward, against torch's own conv / pad / sigmoid;
 8f-5  Trainer.compute_depth_losses (trainer.py:498-526, layers.py:251-269) as a fused metrics call, against the
-      oracle restatement, which is pinned against the reference's own method where /root/reference exists."""
+      oracle restatement, which is pinned against the reference's own method on stored values
+      (tests/golden/reference_interface.json, recorded by tests/golden/make_reference_interface.py)."""
+import json
 import os
-import sys
-import types
 
 import numpy as np
 import pytest
 import torch
 import torch.nn as nn
 
+from helpers import GOLDEN_DIR
 from oracle import view_synthesis as O
 
-REF = "/root/reference"
 
-
-@pytest.mark.skipif(not os.path.isdir(REF), reason="/root/reference is not present on this box")
 def test_oracle_depth_metrics_equal_the_reference_method():
-    for name, attrs in (("tensorboardX", {"SummaryWriter": object}), ("IPython", {"embed": lambda *a, **k: None}),
-                        ("skimage", {}), ("skimage.transform", {})):
-        m = types.ModuleType(name)
-        for k, v in attrs.items():
-            setattr(m, k, v)
-        sys.modules.setdefault(name, m)
-    sys.modules["skimage"].transform = sys.modules["skimage.transform"]
-    sys.dont_write_bytecode = True
-    sys.path.insert(0, REF)
-    try:
-        import trainer as ref_trainer
-    finally:
-        sys.path.remove(REF)
+    """Trainer.compute_depth_losses of the reference on these seeded inputs, as make_reference_interface.py stores it."""
+    with open(os.path.join(GOLDEN_DIR, "reference_interface.json")) as f:
+        losses = json.load(f)["depth_metrics"]
     g = torch.Generator().manual_seed(0)
     depth = torch.rand(3, 1, 48, 160, generator=g) * 40 + 0.5
     gt = torch.rand(3, 1, 375, 1242, generator=g) * 60
     gt[torch.rand(gt.shape, generator=g) < 0.7] = 0            # sparse LiDAR ground truth
-    me = types.SimpleNamespace(depth_metric_names=["de/abs_rel", "de/sq_rel", "de/rms", "de/log_rms", "da/a1", "da/a2", "da/a3"])
-    losses = {}
-    ref_trainer.Trainer.compute_depth_losses(me, {"depth_gt": gt}, {("depth", 0, 0): depth}, losses)
     mine = O.depth_metrics(depth, gt)
-    for i, k in enumerate(me.depth_metric_names):
+    for i, k in enumerate(["de/abs_rel", "de/sq_rel", "de/rms", "de/log_rms", "da/a1", "da/a2", "da/a3"]):
         assert abs(float(mine[i]) - float(losses[k])) <= 1e-6 * abs(float(losses[k])), k
 
 
