@@ -25,6 +25,10 @@ CASES = [
     ("pmask_one_source", 2, 64, 96, [0, "s"], dict(predictive_mask=True, disable_automasking=True)),
     ("pmask_v1", 2, 64, 96, [0, -1, 1], dict(predictive_mask=True, disable_automasking=True, v1_multiscale=True)),
     ("pmask_posecnn", 2, 64, 96, [0, -1, 1], dict(predictive_mask=True, disable_automasking=True, posecnn=True)),
+    # four sources with pose leaves and masks: 4 disparities + 4 x (axisangle, translation) + 4 masks = 16 autograd
+    # leaves, the most md2_scale_tensors takes in its one launch
+    ("pmask_posecnn_4src", 2, 64, 96, [0, -2, -1, 1, 2], dict(predictive_mask=True, disable_automasking=True,
+                                                              posecnn=True)),
 ]
 
 
@@ -125,3 +129,30 @@ def test_kernel_variant_matches_oracle(name, B, H, W, fids, flags):
     assert len(sharp) >= 3 and any(k[0] == "disp" for k in sharp), errs
     if any(k[0] == "axisangle" for k in errs):
         assert any(k[0] in ("axisangle", "translation") for k in sharp), errs
+
+
+def test_scaled_loss_scales_every_gradient_bitwise():
+    """(w * loss).backward() hands w to the call's backward, which multiplies every stored gradient by it in one
+    md2_scale_tensors launch: every leaf kind (disparity, axisangle, translation, mask) of the 16-leaf configuration
+    gets exactly w x the plain gradient."""
+    from monodepth2_b200.fused_loss import LossPlan, view_synthesis_loss
+    name, B, H, W, fids, flags = next(c for c in CASES if c[0] == "pmask_posecnn_4src")
+    inputs, _, leaves, _ = _leaves(B, H, W, fids, flags, 300 + len(name), torch.float32)
+    c_leaves = {k: v.detach().to(DEV).requires_grad_(True) for k, v in leaves.items()}
+    c_outs = {k: c_leaves[k] for k in leaves if k[0] == "disp"}
+    for f in fids[1:]:
+        c_outs[("axisangle", 0, f)], c_outs[("translation", 0, f)] = c_leaves[("axisangle", f)], c_leaves[("translation", f)]
+    c_outs["predictive_mask"] = {("disp", s): c_leaves[("mask", s)] for s in range(4)}
+    losses = view_synthesis_loss(LossPlan(B, H, W, fids, **flags), {k: v.to(DEV) for k, v in inputs.items()}, c_outs)
+    keys = list(c_leaves)
+    assert len(keys) == 16 and {k[0] for k in keys} == {"disp", "axisangle", "translation", "mask"}
+    plain = torch.autograd.grad(losses["loss"], [c_leaves[k] for k in keys], retain_graph=True)
+    w = torch.tensor(-0.7071067811865476, device=DEV)
+    scaled = torch.autograd.grad(w * losses["loss"], [c_leaves[k] for k in keys])
+    for k, a, b in zip(keys, plain, scaled):
+        # bit patterns where the call wrote a gradient; the unused half of a PoseDecoder leaf is autograd's +0 fill
+        # in both runs (w x +0 would be -0 for negative w, an equal value with another bit pattern)
+        nz = a != 0
+        assert bool(nz.any()), k
+        assert torch.equal(b[nz].view(torch.int32), (a[nz] * w).view(torch.int32)), k
+        assert bool((b[~nz] == 0).all()), k

@@ -29,18 +29,29 @@ def test_oracle_depth_metrics_equal_the_reference_method():
         assert abs(float(mine[i]) - float(losses[k])) <= 1e-6 * abs(float(losses[k])), k
 
 
+KITTI_GT, EIGEN_CROP = (375, 1242), (153, 371, 44, 1197)
+
+
 @pytest.mark.gpu
-@pytest.mark.parametrize("shape,sparsity,seed", [((2, 48, 160), 0.7, 1), ((3, 192, 640), 0.95, 2), ((1, 24, 80), 0.0, 3),
-                                                 ((4, 96, 320), 0.5, 4)])
-def test_cuda_depth_metrics_match_oracle(shape, sparsity, seed):
+@pytest.mark.parametrize("shape,sparsity,seed,gt_hw,crop", [
+    pytest.param((2, 48, 160), 0.7, 1, KITTI_GT, EIGEN_CROP, id="shape0-0.7-1"),
+    pytest.param((3, 192, 640), 0.95, 2, KITTI_GT, EIGEN_CROP, id="shape1-0.95-2"),
+    pytest.param((1, 24, 80), 0.0, 3, KITTI_GT, EIGEN_CROP, id="shape2-0.0-3"),
+    pytest.param((4, 96, 320), 0.5, 4, KITTI_GT, EIGEN_CROP, id="shape3-0.5-4"),
+    # gt smaller than the prediction (bilinear down-sampling), gt of odd size, crops reaching past the gt
+    pytest.param((2, 96, 320), 0.3, 5, (48, 160), (10, 40, 20, 150), id="gt_below_pred"),
+    pytest.param((2, 48, 160), 0.5, 6, (37, 123), (20, 375, 50, 1242), id="crop_past_gt"),
+    pytest.param((1, 24, 80), 0.0, 7, (24, 80), (0, 24, 0, 80), id="same_size_full_crop"),
+    pytest.param((3, 12, 40), 0.9, 8, (1, 1242), (0, 1, 44, 1197), id="one_gt_row")])
+def test_cuda_depth_metrics_match_oracle(shape, sparsity, seed, gt_hw, crop):
     from monodepth2_b200 import layers as L
     B, H, W = shape
     g = torch.Generator().manual_seed(seed)
     depth = torch.rand(B, 1, H, W, generator=g) * 60 + 0.05
-    gt = torch.rand(B, 1, 375, 1242, generator=g) * 70 + 0.5
+    gt = torch.rand(B, 1, *gt_hw, generator=g) * 70 + 0.5
     gt[torch.rand(gt.shape, generator=g) < sparsity] = 0
-    ref = O.depth_metrics(depth, gt)
-    got = L.depth_metrics(depth.cuda(), gt.cuda()).cpu()
+    ref = O.depth_metrics(depth, gt, crop)
+    got = L.depth_metrics(depth.cuda(), gt.cuda(), crop).cpu()
     for i, k in enumerate(L.DEPTH_METRIC_NAMES):
         assert abs(float(got[i]) - float(ref[i])) <= 2e-5 * abs(float(ref[i])) + 1e-7, (k, float(got[i]), float(ref[i]))
 
@@ -56,7 +67,8 @@ class _RefConv3x3(nn.Module):          # layers.py:119-136, restated for the com
 
 
 @pytest.mark.gpu
-@pytest.mark.parametrize("B,C,H,W", [(2, 16, 48, 80), (3, 32, 24, 40), (1, 64, 12, 20), (2, 128, 6, 10), (1, 16, 5, 7), (12, 16, 192, 640)])
+@pytest.mark.parametrize("B,C,H,W", [(2, 16, 48, 80), (3, 32, 24, 40), (1, 64, 12, 20), (2, 128, 6, 10), (1, 16, 5, 7), (12, 16, 192, 640),
+                                     (2, 1, 3, 3), (1, 3, 2, 5), (2, 17, 3, 2), (1, 17, 7, 3), (3, 1, 2, 2)])
 def test_cuda_disparity_head_matches_torch(B, C, H, W):
     from monodepth2_b200 import layers as L
     torch.backends.cudnn.allow_tf32 = False
