@@ -57,7 +57,22 @@ typedef struct md2_problem {
                                  trainer.py:127-135): scale slot s of every per-scale array below is pyramid level
                                  scale_level[s], (H >> level, W >> level), smoothness weight 1 / 2^level, and
                                  losses[1 + s] = losses["loss/<level>"].  All zero = levels 0..n-1 */
+  /* ---- element type of the differentiable leaves (md2_dtype; all zero = every leaf fp32).  A bf16 / fp16 leaf is
+   *      widened exactly to fp32 in workspace by one conversion launch at the start of the call, so every result is
+   *      the fp32 call on the upcast leaves, bit for bit.  Losses, cam_T_cam, the side outputs and every grad_* output
+   *      of md2_view_synthesis_loss stay fp32 (the Python wrapper rounds the gradients once to the leaf dtype). ---- */
+  int disp_dtype;                   /* disp[s], every scale */
+  int pose_dtype[MD2_MAX_SRC];      /* source f: T[f], or the axisangle[f] / translation[f] pair (a constant stereo_T
+                                       may stay fp32 while the network's poses are bf16) */
+  int pmask_dtype;                  /* pmask[s], every scale */
 } md2_problem;
+
+/* Element types of md2_problem's *_dtype fields and md2_scale_tensors_typed. */
+typedef enum md2_dtype {
+  MD2_DTYPE_F32 = 0,
+  MD2_DTYPE_BF16 = 1,
+  MD2_DTYPE_F16 = 2
+} md2_dtype;
 
 /* Tensors of one evaluation.  Names follow the reference's dict keys.  Per-scale arrays are indexed by scale SLOT
  * s = 0..num_scales-1; slot s is pyramid level md2_problem.scale_level[s] (= s for the default --scales 0 1 2 3), and
@@ -121,7 +136,8 @@ typedef struct md2_tensors {
 int md2_version(void);
 const char *md2_status_string(int status);
 
-/* Bytes of device scratch the fused call needs for `p`. */
+/* Bytes of device scratch the fused call needs for `p`.  fp32 copies of the reduced-precision leaves are reserved
+ * only when a *_dtype field is non-zero; a dtype outside md2_dtype is MD2_ERR_INVALID_ARGUMENT. */
 int md2_loss_workspace_bytes(const md2_problem *p, size_t *bytes);
 
 /* Fused replacement for Trainer.generate_images_pred (trainer.py:341-391) followed by
@@ -204,6 +220,15 @@ int md2_dispconv_sigmoid(const float *x, const float *weight, const float *bias,
 int md2_dispconv_sigmoid_backward(const float *grad_disp, const float *disp, const float *x, const float *weight,
                                   float *grad_x, float *grad_weight, float *grad_bias,
                                   int batch, int channels, int height, int width, void *stream);
+/* The same head on a bf16 / fp16 feature map (`dtype`, md2_dtype; MD2_DTYPE_F32 selects the fp32 kernels above):
+ * x, disp, grad_disp and grad_x are in `dtype`; weight, bias, grad_weight and grad_bias are fp32.  x is read at 2 bytes
+ * a value and widened exactly; the arithmetic is the fp32 kernels' (weights read in fp32 as stored, not rounded to
+ * bf16 as autocast's conv2d does); disp and grad_x are the fp32 results rounded once to nearest-even. */
+int md2_dispconv_sigmoid_typed(const void *x, const float *weight, const float *bias, void *disp, int dtype,
+                               int batch, int channels, int height, int width, void *stream);
+int md2_dispconv_sigmoid_backward_typed(const void *grad_disp, const void *disp, const void *x, const float *weight,
+                                        void *grad_x, float *grad_weight, float *grad_bias, int dtype,
+                                        int batch, int channels, int height, int width, void *stream);
 
 /* ---- monitoring path (SURVEY.md 8f-5): Trainer.compute_depth_losses, trainer.py:498-526, with
  * compute_depth_errors, layers.py:251-269.  depth = outputs[("depth",0,0)] (B,1,H,W), depth_gt (B,1,Hg,Wg);
@@ -220,6 +245,12 @@ int md2_depth_metrics(const float *depth, const float *depth_gt, float *metrics,
 #define MD2_MAX_SCALE_TENSORS 16
 int md2_scale_tensors(int n_tensors, const float *const *src, float *const *dst, const long long *numel,
                       const float *scale, void *stream);
+/* The same with a destination element type per tensor (dst_dtype[i], md2_dtype; HOST array): dst[i] is the fp32
+ * product src[i] * (*scale) rounded once to nearest-even (an overflow gives +-inf, never a saturated value), so a loss
+ * scale applied before the rounding keeps fp16 gradients that the unscaled product would flush to zero.
+ * Bitwise md2_scale_tensors for an fp32 destination.  One launch. */
+int md2_scale_tensors_typed(int n_tensors, const float *const *src, void *const *dst, const int *dst_dtype,
+                            const long long *numel, const float *scale, void *stream);
 
 /* ---- colour pyramid on the GPU (SURVEY.md 8f-3): replaces the per-frame host work of
  * MonoDataset.preprocess, datasets/mono_dataset.py:57,82-86,98-103 - torchvision Resize with

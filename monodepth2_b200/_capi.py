@@ -11,6 +11,9 @@ import os
 MAX_SCALES = 4
 MAX_SRC = 4
 
+# md2_dtype: element type of a differentiable leaf (md2_problem.*_dtype, md2_scale_tensors_typed, the typed head)
+DTYPE_F32, DTYPE_BF16, DTYPE_F16 = 0, 1, 2
+
 _fp = C.POINTER(C.c_float)
 
 
@@ -23,6 +26,7 @@ class Md2Problem(C.Structure):
         ("want_grad", C.c_int), ("rows_per_segment", C.c_int), ("no_ssim", C.c_int),
         ("posecnn", C.c_int), ("predictive_mask", C.c_int),
         ("scale_level", C.c_int * MAX_SCALES),
+        ("disp_dtype", C.c_int), ("pose_dtype", C.c_int * MAX_SRC), ("pmask_dtype", C.c_int),
     ]
 
 
@@ -76,7 +80,8 @@ SYMBOLS = [
     "md2_smooth_loss", "md2_smooth_loss_backward",
     "md2_pose_to_matrix", "md2_pose_to_matrix_backward",
     "md2_depth_metrics_scratch_bytes", "md2_depth_metrics",
-    "md2_scale_tensors", "md2_dispconv_sigmoid", "md2_dispconv_sigmoid_backward",
+    "md2_scale_tensors", "md2_scale_tensors_typed", "md2_dispconv_sigmoid", "md2_dispconv_sigmoid_backward",
+    "md2_dispconv_sigmoid_typed", "md2_dispconv_sigmoid_backward_typed",
     "md2_resize_plan_create", "md2_resize_plan_destroy", "md2_resize_scratch_bytes", "md2_resize_lanczos_u8",
     "md2_color_jitter_u8",
 ]
@@ -110,6 +115,10 @@ def load_library(path: str = None) -> C.CDLL:
             getattr(lib, name).restype = C.c_int
     lib.md2_scale_tensors.argtypes = [C.c_int, C.POINTER(C.c_void_p), C.POINTER(C.c_void_p), C.POINTER(C.c_longlong),
                                       C.c_void_p, C.c_void_p]
+    lib.md2_scale_tensors_typed.argtypes = [C.c_int, C.POINTER(C.c_void_p), C.POINTER(C.c_void_p), C.POINTER(C.c_int),
+                                            C.POINTER(C.c_longlong), C.c_void_p, C.c_void_p]
+    lib.md2_dispconv_sigmoid_typed.argtypes = [C.c_void_p] * 4 + [C.c_int] * 5 + [C.c_void_p]
+    lib.md2_dispconv_sigmoid_backward_typed.argtypes = [C.c_void_p] * 7 + [C.c_int] * 5 + [C.c_void_p]
     lib.md2_depth_metrics_scratch_bytes.argtypes = [C.c_int, C.c_int, C.c_int, C.POINTER(C.c_size_t)]
     lib.md2_depth_metrics.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_size_t] + [C.c_int] * 9 + [C.c_void_p]
     lib.md2_resize_plan_destroy.restype = None

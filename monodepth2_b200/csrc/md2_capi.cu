@@ -10,14 +10,14 @@ namespace md2 {
 cudaError_t debug_set_sink(const DebugSink* host_copy);
 cudaError_t debug_oob_count(unsigned long long* count, int reset);
 #endif
-cudaError_t launch_view_synthesis_loss(const Params& P, cudaStream_t stream);
+cudaError_t launch_view_synthesis_loss(const Params& P, const Widen& Wd, cudaStream_t stream);
 cudaError_t profile_enable(bool on);
 cudaError_t profile_march_ms(float* ms);
 }
 
 extern "C" {
 
-int md2_version(void) { return 100; }
+int md2_version(void) { return 101; }
 
 const char* md2_status_string(int status) {
   switch (status) {
@@ -46,7 +46,9 @@ int md2_view_synthesis_loss(const md2_problem* p, const md2_tensors* t, void* wo
   md2::Params P;
   st = md2::fill_params(p, t, workspace, &P);
   if (st != MD2_OK) return st;
-  const cudaError_t e = md2::launch_view_synthesis_loss(P, (cudaStream_t)stream);
+  md2::Widen Wd;
+  md2::fill_widen(p, workspace, &P, &Wd);
+  const cudaError_t e = md2::launch_view_synthesis_loss(P, Wd, (cudaStream_t)stream);
   return e == cudaSuccess ? MD2_OK : MD2_ERR_CUDA;
 }
 

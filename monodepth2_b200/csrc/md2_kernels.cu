@@ -15,6 +15,8 @@
 // adjoint needs two rows later sit in a thread-private shared-memory ring.  No block-level
 // synchronisation, no tensor cores (the path is gather/stream work, BASELINE.json).
 #include <cuda.h>
+#include <cuda_bf16.h>
+#include <cuda_fp16.h>
 #include <cuda_runtime.h>
 #include <stdint.h>
 #include <stdlib.h>
@@ -1163,6 +1165,19 @@ __global__ void __launch_bounds__(256) md2_u8_to_f32(Params P) {
   }
 }
 
+// bf16 / fp16 leaves (md2_problem::*_dtype, planned by fill_widen): every reduced-precision disparity, mask and pose
+// leaf widened exactly to fp32 in workspace, one launch for all of them (blockIdx.y = job).  It runs on the caller's
+// stream before anything else, so the prologue, the side-stream kernels and the marching kernel all read fp32 copies.
+__global__ void __launch_bounds__(256) md2_widen(Widen Wd) {
+  const WidenJob& j = Wd.job[blockIdx.y];
+  const long long step = (long long)gridDim.x * blockDim.x;
+  for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < j.n; i += step) {
+    const long long si = j.row ? (i / j.row) * j.stride + i % j.row : i;
+    j.dst[i] = j.dtype == MD2_DTYPE_BF16 ? __bfloat162float(((const __nv_bfloat16*)j.src)[si])
+                                         : __half2float(((const __half*)j.src)[si]);
+  }
+}
+
 static cudaError_t launch_float_entry(const Params& P, cudaStream_t stream);
 
 // The fork / join events and the side streams are shared by every call on a device: the enqueue of one call (a few
@@ -1170,8 +1185,15 @@ static cudaError_t launch_float_entry(const Params& P, cudaStream_t stream);
 // different streams - cannot interleave their event records and waits.  The GPU work itself is not serialised by this.
 static std::mutex g_enqueue_mu;
 
-cudaError_t launch_view_synthesis_loss(const Params& P, cudaStream_t stream) {
+cudaError_t launch_view_synthesis_loss(const Params& P, const Widen& Wd, cudaStream_t stream) {
   std::lock_guard<std::mutex> enqueue_lock(g_enqueue_mu);
+  if (Wd.n > 0) {
+    long long bx = (Wd.max_n + 255) / 256;
+    if (bx > 1184) bx = 1184;                     // 8 blocks per SM, grid-stride beyond
+    md2_widen<<<dim3((unsigned)bx, Wd.n), 256, 0, stream>>>(Wd);
+    const cudaError_t e = cudaGetLastError();
+    if (e != cudaSuccess) return e;
+  }
 #ifndef MD2_DBG_DEVICE
   static const bool cvt_on = !(getenv("MD2_U8_CONVERT") && atoi(getenv("MD2_U8_CONVERT")) == 0);
   if (P.tgt8 && cvt_on) {

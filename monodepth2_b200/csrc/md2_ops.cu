@@ -2,6 +2,8 @@
 // (include/md2_loss.h, "per-layer entry points").  These keep the reference's unfused
 // call graph working (trainer.py calling BackprojectDepth -> Project3D -> grid_sample ->
 // SSIM ...); the fused md2_view_synthesis_loss is the fast path.
+#include <cuda_bf16.h>
+#include <cuda_fp16.h>
 #include <cuda_runtime.h>
 #include <math.h>
 
@@ -360,6 +362,35 @@ __global__ void k_scale_tensors(ScaleArgs a, const float* __restrict__ scale) {
     if (j + k < a.numel[i]) d[j + k] = __ldg(s + j + k) * g;
 }
 
+// md2_scale_tensors with a destination type per tensor: the fp32 product, rounded once (round-to-nearest-even; an
+// overflow rounds to +-inf, which GradScaler's found-inf check relies on)
+struct ScaleTypedArgs {
+  const float* src[MD2_MAX_SCALE_TENSORS];
+  void* dst[MD2_MAX_SCALE_TENSORS];
+  long long start[MD2_MAX_SCALE_TENSORS + 1];
+  long long numel[MD2_MAX_SCALE_TENSORS];
+  int dtype[MD2_MAX_SCALE_TENSORS];
+  int n;
+};
+__global__ void k_scale_tensors_typed(ScaleTypedArgs a, const float* __restrict__ scale) {
+  const long long q = ((long long)blockIdx.x * blockDim.x + threadIdx.x) * 4;
+  if (q >= a.start[a.n]) return;
+  int i = 0;
+  while (i + 1 < a.n && q >= a.start[i + 1]) ++i;
+  const long long j = q - a.start[i];
+  const float g = __ldg(scale);
+  const float* s = a.src[i];
+  const int dt = a.dtype[i];
+#pragma unroll
+  for (int k = 0; k < 4; ++k) {
+    if (j + k >= a.numel[i]) break;
+    const float v = __ldg(s + j + k) * g;
+    if (dt == MD2_DTYPE_BF16) ((__nv_bfloat16*)a.dst[i])[j + k] = __float2bfloat16_rn(v);
+    else if (dt == MD2_DTYPE_F16) ((__half*)a.dst[i])[j + k] = __float2half_rn(v);
+    else ((float*)a.dst[i])[j + k] = v;
+  }
+}
+
 extern "C" {
 
 int md2_disp_to_depth(const float* disp, float min_depth, float max_depth, float* scaled_disp, float* depth,
@@ -504,6 +535,28 @@ int md2_scale_tensors(int n_tensors, const float* const* src, float* const* dst,
   if (total == 0) return MD2_OK;
   const long long threads = total / 4;
   k_scale_tensors<<<(unsigned)((threads + kT - 1) / kT), kT, 0, (cudaStream_t)stream>>>(a, scale);
+  return rc(cudaGetLastError());
+}
+
+int md2_scale_tensors_typed(int n_tensors, const float* const* src, void* const* dst, const int* dst_dtype,
+                            const long long* numel, const float* scale, void* stream) {
+  if (n_tensors < 1 || n_tensors > MD2_MAX_SCALE_TENSORS || !src || !dst || !dst_dtype || !numel || !scale)
+    return MD2_ERR_INVALID_ARGUMENT;
+  ScaleTypedArgs a;
+  long long total = 0;
+  for (int i = 0; i < n_tensors; ++i) {
+    const int d = dst_dtype[i];
+    if (!src[i] || !dst[i] || numel[i] < 0) return MD2_ERR_INVALID_ARGUMENT;
+    if (d != MD2_DTYPE_F32 && d != MD2_DTYPE_BF16 && d != MD2_DTYPE_F16) return MD2_ERR_INVALID_ARGUMENT;
+    a.src[i] = src[i]; a.dst[i] = dst[i]; a.dtype[i] = d; a.start[i] = total;
+    total += (numel[i] + 3) / 4 * 4;
+  }
+  a.start[n_tensors] = total;
+  a.n = n_tensors;
+  for (int i = 0; i < n_tensors; ++i) a.numel[i] = numel[i];
+  if (total == 0) return MD2_OK;
+  const long long threads = total / 4;
+  k_scale_tensors_typed<<<(unsigned)((threads + kT - 1) / kT), kT, 0, (cudaStream_t)stream>>>(a, scale);
   return rc(cudaGetLastError());
 }
 

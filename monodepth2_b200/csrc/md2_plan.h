@@ -23,7 +23,25 @@ struct Layout {
   size_t mid_off, gmidc_off;                       // posecnn
   size_t pm_off[kMaxScales], gpm_off[kMaxScales];  // predictive mask
   size_t cvt_img_off[1 + kMaxSrc], cvt_col_off[kMaxScales];   // uint8 entry: frames / pyramid as planar float
+  size_t wd_disp_off[kMaxScales], wd_pm_off[kMaxScales];      // bf16 / fp16 leaves widened to fp32 (md2_widen)
+  size_t wd_pose_off[kMaxSrc];                                // T (16 B floats) or axisangle | translation (3 B each)
   size_t total;
+};
+
+// bf16 / fp16 leaves (md2_problem::*_dtype): md2_widen copies each into an fp32 workspace buffer before the prologue,
+// and the Params pointers are redirected to the copies, so no kernel downstream knows the leaves were narrower.
+// Element i of a job reads src[(i / row) * stride + i % row] (row = 0: src[i]).
+constexpr int kMaxWiden = 2 * kMaxScales + 2 * kMaxSrc;
+struct WidenJob {
+  const void* src;
+  float* dst;
+  long long n;
+  int row, stride, dtype;
+};
+struct Widen {
+  int n;                 // jobs; 0 = nothing to launch (every leaf fp32)
+  long long max_n;       // largest job, sizes the grid
+  WidenJob job[kMaxWiden];
 };
 
 // Pyramid level of scale slot s: md2_problem::scale_level when given (strictly ascending, trainer.py:345,413 iterate
@@ -34,8 +52,12 @@ inline bool custom_levels(const md2_problem* p) {
 }
 inline int level_of(const md2_problem* p, int s) { return custom_levels(p) ? p->scale_level[s] : s; }
 
+inline bool dtype_ok(int d) { return d == MD2_DTYPE_F32 || d == MD2_DTYPE_BF16 || d == MD2_DTYPE_F16; }
+
 inline int validate(const md2_problem* p) {
   if (!p) return MD2_ERR_INVALID_ARGUMENT;
+  if (!dtype_ok(p->disp_dtype) || !dtype_ok(p->pmask_dtype)) return MD2_ERR_INVALID_ARGUMENT;
+  for (int f = 0; f < MD2_MAX_SRC; ++f) if (!dtype_ok(p->pose_dtype[f])) return MD2_ERR_INVALID_ARGUMENT;
   if (p->batch < 1 || p->height < 4 || p->width < 4) return MD2_ERR_INVALID_ARGUMENT;
   if (p->num_scales < 1 || p->num_scales > MD2_MAX_SCALES) return MD2_ERR_INVALID_ARGUMENT;
   if (p->num_src < 1 || p->num_src > MD2_MAX_SRC) return MD2_ERR_INVALID_ARGUMENT;
@@ -93,6 +115,17 @@ inline Layout make_layout(const md2_problem* p) {
     if (lv == 0) continue;                      // level 0 = the converted target frame
     L.cvt_col_off[s] = off; off = align_up(off + B * 3 * (H >> lv) * (W >> lv) * sizeof(float), 256);
   }
+  // fp32 copies of reduced-precision leaves, after everything else: an all-fp32 problem keeps its layout and size
+  for (int s = 0; s < p->num_scales; ++s) {
+    const int lv = level_of(p, s);
+    const size_t plane = (H >> lv) * (W >> lv);
+    if (p->disp_dtype != MD2_DTYPE_F32) { L.wd_disp_off[s] = off; off = align_up(off + B * plane * sizeof(float), 256); }
+    if (p->predictive_mask && p->pmask_dtype != MD2_DTYPE_F32) {
+      L.wd_pm_off[s] = off; off = align_up(off + B * p->num_src * plane * sizeof(float), 256);
+    }
+  }
+  for (int f = 0; f < p->num_src; ++f)
+    if (p->pose_dtype[f] != MD2_DTYPE_F32) { L.wd_pose_off[f] = off; off = align_up(off + B * 16 * sizeof(float), 256); }
   L.total = off;
   return L;
 }
@@ -244,6 +277,37 @@ inline int fill_params(const md2_problem* p, const md2_tensors* t, void* workspa
   P->tgt4 = (float*)(ws + L.tgt4_off);
   for (int f = 0; f < p->num_src; ++f) P->src4[f] = (float*)(ws + L.src4_off[f]);
   return MD2_OK;
+}
+
+// After fill_params: lists the reduced-precision leaves in `Wd` and points `P` at their fp32 workspace copies.
+inline void fill_widen(const md2_problem* p, void* workspace, Params* P, Widen* Wd) {
+  memset(Wd, 0, sizeof(*Wd));
+  const Layout L = make_layout(p);
+  char* ws = (char*)workspace;
+  auto add = [&](const void* src, size_t off, long long n, int row, int stride, int dtype) -> float* {
+    WidenJob& j = Wd->job[Wd->n++];
+    j.src = src; j.dst = (float*)(ws + off); j.n = n; j.row = row; j.stride = stride; j.dtype = dtype;
+    if (n > Wd->max_n) Wd->max_n = n;
+    return j.dst;
+  };
+  const long long B = p->batch;
+  for (int s = 0; s < p->num_scales; ++s) {
+    const long long plane = (long long)(p->height >> P->lvl[s]) * (p->width >> P->lvl[s]);
+    if (p->disp_dtype != MD2_DTYPE_F32) P->disp[s] = add(P->disp[s], L.wd_disp_off[s], B * plane, 0, 0, p->disp_dtype);
+    if (P->pmask_on && p->pmask_dtype != MD2_DTYPE_F32)
+      P->pmask[s] = add(P->pmask[s], L.wd_pm_off[s], B * p->num_src * plane, 0, 0, p->pmask_dtype);
+  }
+  for (int f = 0; f < p->num_src; ++f) {
+    const int d = p->pose_dtype[f];
+    if (d == MD2_DTYPE_F32) continue;
+    if (P->aa[f]) {         // pose leaves: 3 values per sample, pose_stride apart; the copies are packed (stride 3)
+      P->aa[f] = add(P->aa[f], L.wd_pose_off[f], 3 * B, 3, P->pose_stride[f], d);
+      P->tr[f] = add(P->tr[f], L.wd_pose_off[f] + 3 * B * sizeof(float), 3 * B, 3, P->pose_stride[f], d);
+      P->pose_stride[f] = 3;
+    } else {
+      P->Tm[f] = add(P->Tm[f], L.wd_pose_off[f], 16 * B, 0, 0, d);
+    }
+  }
 }
 
 }  // namespace md2

@@ -30,6 +30,31 @@ def _check_f32_cuda(t: torch.Tensor, name: str, shape=None) -> torch.Tensor:
     return t.contiguous()
 
 
+# element types a differentiable leaf may have (md2_problem.disp_dtype / pose_dtype / pmask_dtype)
+_LEAF_DTYPES = {torch.float32: _capi.DTYPE_F32, torch.bfloat16: _capi.DTYPE_BF16, torch.float16: _capi.DTYPE_F16}
+
+
+def _check_leaf_cuda(t: torch.Tensor, name: str, shape=None) -> torch.Tensor:
+    """A differentiable leaf: float32, bfloat16 or float16 (what the networks give under torch.autocast).  A narrower
+    leaf is widened exactly inside the call; nothing here converts it."""
+    if not t.is_cuda:
+        raise RuntimeError("%s must be a CUDA tensor (the fused loss has no CPU path)" % name)
+    if t.dtype not in _LEAF_DTYPES:
+        raise RuntimeError("%s must be float32, bfloat16 or float16, got %s" % (name, t.dtype))
+    if shape is not None and tuple(t.shape) != tuple(shape):
+        raise RuntimeError("%s has shape %s, expected %s" % (name, tuple(t.shape), tuple(shape)))
+    return t.contiguous()
+
+
+def _one_dtype(tensors: Sequence, names: Sequence[str], what: str) -> int:
+    """The md2_dtype shared by ``tensors``; a mix raises, naming each tensor and its dtype."""
+    dts = [t.dtype for t in tensors]
+    if len(set(dts)) > 1 or any(d not in _LEAF_DTYPES for d in dts):
+        raise RuntimeError("%s must share one dtype out of float32, bfloat16 and float16, got %s"
+                           % (what, ", ".join("%s %s" % (n, d) for n, d in zip(names, dts))))
+    return _LEAF_DTYPES[dts[0]] if dts else _capi.DTYPE_F32
+
+
 def _check_u8_cuda(t: torch.Tensor, name: str, B: int, H: int, W: int, hwc: bool) -> torch.Tensor:
     if not t.is_cuda:
         raise RuntimeError("%s must be a CUDA tensor (the fused loss has no CPU path)" % name)
@@ -104,8 +129,11 @@ class LossPlan:
                    posecnn=(getattr(opt, "pose_model_type", "separate_resnet") == "posecnn"),
                    predictive_mask=getattr(opt, "predictive_mask", False), **kw)
 
-    def problem(self, want_grad: bool) -> Md2Problem:
-        return Md2Problem(batch=self.batch_size, height=self.height, width=self.width,
+    def problem(self, want_grad: bool, dtypes=None) -> Md2Problem:
+        """``dtypes`` = (disp_dtype, (pose_dtype per source), pmask_dtype) of md2_problem; None = every leaf fp32."""
+        disp_dt, pose_dt, pmask_dt = dtypes or (0, (), 0)
+        pose = (C.c_int * _capi.MAX_SRC)(*pose_dt)
+        return Md2Problem(disp_dtype=disp_dt, pose_dtype=pose, pmask_dtype=pmask_dt,batch=self.batch_size, height=self.height, width=self.width,
                           num_scales=len(self.scales), num_src=self.n_src, automask=int(self.automask),
                           avg_reprojection=int(self.avg_reprojection), align_corners=int(self.align_corners),
                           min_depth=self.min_depth, max_depth=self.max_depth,
@@ -126,12 +154,14 @@ class LossPlan:
         """Index of pyramid level ``level`` in the per-scale arrays of the C ABI."""
         return self.scales.index(level)
 
-    def workspace(self, device: torch.device) -> torch.Tensor:
-        key = (device.type, device.index)
+    def workspace(self, device: torch.device, dtypes=None) -> torch.Tensor:
+        """The call's device scratch; reduced-precision leaves (``dtypes``, see ``problem``) add their fp32 copies."""
+        narrow = dtypes is not None and (dtypes[0] or any(dtypes[1]) or dtypes[2])
+        key = (device.type, device.index) + ((dtypes,) if narrow else ())
         ws = self._workspace.get(key)
         if ws is None:
             n = C.c_size_t(0)
-            p = self.problem(True)
+            p = self.problem(True, dtypes)
             _capi.check(self.lib, self.lib.md2_loss_workspace_bytes(C.byref(p), C.byref(n)), "md2_loss_workspace_bytes")
             ws = torch.empty(n.value, dtype=torch.uint8, device=device)
             self._workspace[key] = ws
@@ -167,8 +197,8 @@ class _ViewSynthesisLossFn(torch.autograd.Function):
         def pose_leaf(x, name):
             # (B,3) / (B,1,3) view whose 3 components are adjacent; any batch stride (e.g. the [:, 0] view of
             # PoseDecoder's (B,2,1,3) output, pose_decoder.py:49-54)
-            if not x.is_cuda or x.dtype != torch.float32:
-                raise RuntimeError("%s must be a CUDA float32 tensor" % name)
+            if not x.is_cuda or x.dtype not in _LEAF_DTYPES:
+                raise RuntimeError("%s must be a CUDA float32, bfloat16 or float16 tensor, got %s" % (name, x.dtype))
             if x.numel() != B * 3 or x.shape[0] != B or x.shape[-1] != 3:
                 raise RuntimeError("%s has shape %s, expected (%d,1,3)" % (name, tuple(x.shape), B))
             if x.stride(-1) != 1 or (B > 1 and x.stride(0) < 3):
@@ -186,6 +216,13 @@ class _ViewSynthesisLossFn(torch.autograd.Function):
             t.target = ptr(_check_f32_cuda(target, "target", (B, 3, H, W)))
         cam_T = [None] * F
         grad_first, grad_second = [None] * F, [None] * F
+        # one dtype for all disparities, one for all masks, one per source (T, or the axisangle / translation pair)
+        disp_dt = _one_dtype(disps, ["disp[%d]" % s for s in range(S)], "the disparities")
+        mask_dt = _one_dtype(masks, ["predictive_mask[%d]" % s for s in range(S)], "the predictive masks")
+        pose_dt = [_one_dtype([x for x in (firsts[i], seconds[i]) if x is not None],
+                              ["axisangle[%d]" % i, "translation[%d]" % i] if pose_invert[i] is not None else ["T[%d]" % i],
+                              "the pose leaves of source %d" % i) for i in range(F)]
+        dtypes = (disp_dt, tuple(pose_dt), mask_dt)
         for i in range(F):
             if u8:
                 t.source_u8[i] = ptr(_check_u8_cuda(sources[i], "source[%d]" % i, B, H, W, hwc))
@@ -193,7 +230,7 @@ class _ViewSynthesisLossFn(torch.autograd.Function):
                 t.source[i] = ptr(_check_f32_cuda(sources[i], "source[%d]" % i, (B, 3, H, W)))
             t.pose_requires_grad[i] = int(bool(pose_grad[i]))
             if pose_invert[i] is None:
-                t.T[i] = ptr(_check_f32_cuda(firsts[i], "T[%d]" % i, (B, 4, 4)))
+                t.T[i] = ptr(_check_leaf_cuda(firsts[i], "T[%d]" % i, (B, 4, 4)))
                 if want_grad:
                     grad_first[i] = torch.empty((B, 4, 4), dtype=torch.float32, device=dev)
                     t.grad_T[i] = ptr(grad_first[i])
@@ -216,7 +253,7 @@ class _ViewSynthesisLossFn(torch.autograd.Function):
         grad_mask = [None] * S
         for s in range(S):
             hs, ws = H >> plan.scales[s], W >> plan.scales[s]
-            t.disp[s] = ptr(_check_f32_cuda(disps[s], "disp[%d]" % s, (B, 1, hs, ws)))
+            t.disp[s] = ptr(_check_leaf_cuda(disps[s], "disp[%d]" % s, (B, 1, hs, ws)))
             if u8:
                 t.color_u8[s] = ptr(_check_u8_cuda(colors[s], "color[%d]" % s, B, hs, ws, hwc))
             else:
@@ -232,7 +269,7 @@ class _ViewSynthesisLossFn(torch.autograd.Function):
                 grad_disp.append(g)
                 t.grad_disp[s] = ptr(g)
             if plan.predictive_mask:
-                t.pmask[s] = ptr(_check_f32_cuda(masks[s], "predictive_mask[%d]" % s, (B, F, hs, ws)))
+                t.pmask[s] = ptr(_check_leaf_cuda(masks[s], "predictive_mask[%d]" % s, (B, F, hs, ws)))
                 if want_grad and ctx.needs_input_grad[_ViewSynthesisLossFn.N_FIXED + S + 2 * F + s]:
                     g = torch.empty((B, F, hs, ws), dtype=torch.float32, device=dev)
                     grad_mask[s] = g
@@ -260,8 +297,8 @@ class _ViewSynthesisLossFn(torch.autograd.Function):
             side["_cam_T_cam"] = cam_T
         losses = torch.empty(MAX_SCALES + 1, dtype=torch.float32, device=dev)
         t.losses = ptr(losses)
-        ws_buf = plan.workspace(dev)
-        p = plan.problem(want_grad)
+        ws_buf = plan.workspace(dev, dtypes)
+        p = plan.problem(want_grad, dtypes)
         with torch.cuda.device(dev):
             stream = torch.cuda.current_stream().cuda_stream
             st = plan.lib.md2_view_synthesis_loss(C.byref(p), C.byref(t), ws_buf.data_ptr(), ws_buf.numel(),
@@ -275,6 +312,7 @@ class _ViewSynthesisLossFn(torch.autograd.Function):
         ctx.have = [(grad_first[i] is not None, grad_second[i] is not None) for i in range(F)]
         ctx.have_mask = [g is not None for g in grad_mask]
         ctx.n_leaves = len(leaves)
+        ctx.leaf_dtypes = [x.dtype if x is not None else None for x in leaves]
         if want_grad:
             ctx.save_for_backward(*grad_disp, *[g for g in grad_first if g is not None],
                                   *[g for g in grad_second if g is not None],
@@ -290,7 +328,9 @@ class _ViewSynthesisLossFn(torch.autograd.Function):
         saved = list(ctx.saved_tensors)
         S, F = ctx.S, ctx.F
         n0 = _ViewSynthesisLossFn.N_FIXED
-        # every stored gradient times the incoming scalar, all tensors in ONE launch (md2_scale_tensors)
+        # every stored gradient times the incoming scalar, all tensors in ONE launch (md2_scale_tensors); a bf16 / fp16
+        # leaf gets the fp32 product rounded once to its dtype (md2_scale_tensors_typed): the scalar - a GradScaler
+        # scale, a loss weight - is applied before the rounding, so scaled fp16 gradients do not flush to zero
         want = []           # (slot in the result tuple, stored gradient, shape)
         for s in range(S):
             if ctx.needs_input_grad[n0 + s]:
@@ -313,15 +353,22 @@ class _ViewSynthesisLossFn(torch.autograd.Function):
         out = [None] * (n0 + ctx.n_leaves)
         if want:
             n = len(want)
-            res = [torch.empty_like(w[1]) for w in want]
+            dts = [ctx.leaf_dtypes[w[0] - n0] for w in want]
+            res = [torch.empty_like(w[1], dtype=d) for w, d in zip(want, dts)]
             g = g_total.detach().to(torch.float32).contiguous()
             src = (C.c_void_p * n)(*[w[1].data_ptr() for w in want])
             dst = (C.c_void_p * n)(*[r.data_ptr() for r in res])
             cnt = (C.c_longlong * n)(*[w[1].numel() for w in want])
             with torch.cuda.device(g.device):
-                st = ctx.lib.md2_scale_tensors(n, src, dst, cnt, g.data_ptr(),
-                                               C.c_void_p(torch.cuda.current_stream().cuda_stream))
-            _capi.check(ctx.lib, st, "md2_scale_tensors")
+                stream = C.c_void_p(torch.cuda.current_stream().cuda_stream)
+                if all(d == torch.float32 for d in dts):
+                    name = "md2_scale_tensors"
+                    st = ctx.lib.md2_scale_tensors(n, src, dst, cnt, g.data_ptr(), stream)
+                else:
+                    name = "md2_scale_tensors_typed"
+                    dt = (C.c_int * n)(*[_LEAF_DTYPES[d] for d in dts])
+                    st = ctx.lib.md2_scale_tensors_typed(n, src, dst, dt, cnt, g.data_ptr(), stream)
+            _capi.check(ctx.lib, st, name)
             for w, r in zip(want, res):
                 out[w[0]] = r.reshape(w[2])
         return tuple(out)
@@ -454,10 +501,17 @@ def view_synthesis_loss(plan: LossPlan, inputs: Dict, outputs: Dict,
     return losses
 
 
+def _widened(x: torch.Tensor) -> torch.Tensor:
+    return x.float() if x.dtype in (torch.bfloat16, torch.float16) else x
+
+
 def _view_synthesis_loss_v1_multiscale(plan: LossPlan, inputs: Dict, outputs: Dict, noise, side):
     """--v1_multiscale: one single-scale fused call per pyramid level (source_scale = scale)."""
     losses: Dict[str, torch.Tensor] = {}
     total = 0
+    # the pose tensors feed every per-level call: a bf16 / fp16 one is widened once, in the graph, so that autograd sums
+    # the per-level gradients in fp32 and rounds the sum once to the leaf's dtype, as a single call would
+    shared: Dict = {}
     for i, s in enumerate(plan.scales):
         sp = plan._scale_plans[i]
         ins = {("K", 0): inputs[("K", s)], ("inv_K", 0): inputs[("inv_K", s)]}
@@ -470,7 +524,7 @@ def _view_synthesis_loss_v1_multiscale(plan: LossPlan, inputs: Dict, outputs: Di
             if f != "s":       # the matrix if the caller built it, else the pose leaves (T is then built in the call)
                 for key in (("cam_T_cam", 0, f), ("axisangle", 0, f), ("translation", 0, f)):
                     if key in outputs:
-                        outs[key] = outputs[key]
+                        outs[key] = shared.setdefault(key, _widened(outputs[key]))
         if plan.predictive_mask:      # not up-sampled under --v1_multiscale (trainer.py:450)
             outs["predictive_mask"] = {("disp", 0): outputs["predictive_mask"][("disp", s)]}
         sub_side = None

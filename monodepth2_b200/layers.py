@@ -4,8 +4,9 @@ Same class names, constructor arguments, call signatures and tensor conventions 
 /root/reference/layers.py, so ``trainer.py``'s ``from layers import *`` (trainer.py:22)
 can point here unchanged.  Every op below launches a hand-written sm_100a kernel of
 libmd2loss.so through the C ABI (include/md2_loss.h); autograd is wired with
-``torch.autograd.Function``.  Inputs must be CUDA float32 tensors: there is no
-PyTorch/CPU fallback, a missing library or a CPU tensor raises.
+``torch.autograd.Function``.  Inputs must be CUDA float32 tensors (the disparity head
+also takes a bfloat16 / float16 feature map): there is no PyTorch/CPU fallback, a missing
+library or a CPU tensor raises.
 
 The fused fast path is ``monodepth2_b200.fused_loss`` (one call replaces
 generate_images_pred + compute_losses); these per-layer ops keep the reference's
@@ -307,18 +308,36 @@ def get_smooth_loss(disp, img):
 
 
 # ------------------------------------------------------------------ decoder tail feeding the path (SURVEY.md 8f-4)
+_HEAD_DTYPES = {torch.float32: _capi.DTYPE_F32, torch.bfloat16: _capi.DTYPE_BF16, torch.float16: _capi.DTYPE_F16}
+
+
+def _head_map(t: torch.Tensor, name: str, dtype=None) -> torch.Tensor:
+    """A feature-map-side tensor of the head: CUDA, float32 / bfloat16 / float16 (``dtype`` when given)."""
+    if not isinstance(t, torch.Tensor) or not t.is_cuda:
+        raise RuntimeError("%s must be a CUDA tensor (monodepth2_b200.layers has no CPU path)" % name)
+    if t.dtype not in _HEAD_DTYPES or (dtype is not None and t.dtype != dtype):
+        raise RuntimeError("%s must be %s, got %s" % (name, dtype or "float32, bfloat16 or float16", t.dtype))
+    return t.contiguous()
+
+
 class _DispHead(torch.autograd.Function):
-    """sigmoid(Conv3x3(C -> 1)(x)) in one pass (md2_dispconv_sigmoid): networks/depth_decoder.py:60-63."""
+    """sigmoid(Conv3x3(C -> 1)(x)) in one pass (md2_dispconv_sigmoid_typed): networks/depth_decoder.py:60-63.
+
+    ``x`` may be float32, bfloat16 or float16 (what the decoder gives under ``torch.autocast``); ``disp`` and the
+    gradient of ``x`` come back in ``x``'s dtype, the weight and bias gradients in float32.  A reduced-precision ``x`` is
+    read at 2 bytes a value and widened exactly; weights and bias are read in float32 as stored - more accurate than
+    autocast's own ``conv2d``, which rounds the weights to bfloat16 - and ``disp`` is the float32 result rounded once
+    (nearest-even): bitwise the float32 head on ``x.float()``, then ``.to(x.dtype)``."""
 
     @staticmethod
     def forward(ctx, x, weight, bias):
-        x, w, b = _f32c(x, "x"), _f32c(weight, "weight"), _f32c(bias, "bias")
+        x, w, b = _head_map(x, "x"), _f32c(weight, "weight"), _f32c(bias, "bias")
         B, Cc, H, W = x.shape
         if tuple(w.shape) != (1, Cc, 3, 3) or b.numel() != 1:
             raise RuntimeError("DispConvSigmoid: weight %s / bias %s do not fit x %s" % (tuple(w.shape), tuple(b.shape), tuple(x.shape)))
-        disp = torch.empty((B, 1, H, W), dtype=torch.float32, device=x.device)
-        _call("md2_dispconv_sigmoid", x.device, _p(x), _p(w), _p(b), _p(disp), C.c_int(B), C.c_int(Cc), C.c_int(H),
-              C.c_int(W), _stream(x))
+        disp = torch.empty((B, 1, H, W), dtype=x.dtype, device=x.device)
+        _call("md2_dispconv_sigmoid_typed", x.device, _p(x), _p(w), _p(b), _p(disp), C.c_int(_HEAD_DTYPES[x.dtype]),
+              C.c_int(B), C.c_int(Cc), C.c_int(H), C.c_int(W), _stream(x))
         ctx.save_for_backward(x, w, disp)
         return disp
 
@@ -326,15 +345,16 @@ class _DispHead(torch.autograd.Function):
     @torch.autograd.function.once_differentiable
     def backward(ctx, g):
         x, w, disp = ctx.saved_tensors
-        g = _f32c(g, "grad_disp")
+        g = _head_map(g, "grad_disp", x.dtype)
         B, Cc, H, W = x.shape
         gx = torch.empty_like(x) if ctx.needs_input_grad[0] else None
         need_w = ctx.needs_input_grad[1] or ctx.needs_input_grad[2]
         gw = torch.empty_like(w) if need_w else None
         gb = torch.empty(1, dtype=torch.float32, device=x.device) if need_w else None
-        _call("md2_dispconv_sigmoid_backward", x.device, _p(g), _p(disp), _p(x), _p(w),
+        _call("md2_dispconv_sigmoid_backward_typed", x.device, _p(g), _p(disp), _p(x), _p(w),
               _p(gx) if gx is not None else None, _p(gw) if gw is not None else None,
-              _p(gb) if gb is not None else None, C.c_int(B), C.c_int(Cc), C.c_int(H), C.c_int(W), _stream(x))
+              _p(gb) if gb is not None else None, C.c_int(_HEAD_DTYPES[x.dtype]), C.c_int(B), C.c_int(Cc), C.c_int(H),
+              C.c_int(W), _stream(x))
         return gx, (gw if ctx.needs_input_grad[1] else None), (gb if ctx.needs_input_grad[2] else None)
 
 
@@ -356,7 +376,8 @@ class DispConvSigmoid(nn.Module):
 def fuse_disp_heads(depth_decoder):
     """Replace every ``("dispconv", s)`` Conv3x3 of a reference DepthDecoder by a DispConvSigmoid that shares its
     parameters, and its trailing ``sigmoid`` by the identity: ``decoder.forward`` (depth_decoder.py:48-65) then hands
-    ``outputs[("disp", s)]`` straight from the fused head.  Returns the decoder."""
+    ``outputs[("disp", s)]`` straight from the fused head.  Under ``torch.autocast`` the decoder's feature maps are
+    bfloat16 / float16 and so are the disparities it hands on (see ``_DispHead``).  Returns the decoder."""
     for key, mod in list(depth_decoder.convs.items()):
         if not (isinstance(key, tuple) and key[0] == "dispconv"):
             continue
