@@ -230,6 +230,24 @@ int md2_dispconv_sigmoid_backward_typed(const void *grad_disp, const void *disp,
                                         void *grad_x, float *grad_weight, float *grad_bias, int dtype,
                                         int batch, int channels, int height, int width, void *stream);
 
+/* ---- decoder stages (SURVEY.md 8f-4): the input of every ConvBlock of DepthDecoder.forward,
+ * networks/depth_decoder.py:48-65 - upsample (layers.py:196-199), torch.cat and the ReflectionPad2d(1) of Conv3x3
+ * (layers.py:106-136) - in one pass:
+ *   out = ReflectionPad2d(1)(cat([nearest_up(x, up), skip], dim=1))
+ * x (B,Cx,h,w); skip (B,Cs,up*h,up*w), or NULL with Cs = 0; out (B,Cx+Cs,up*h+2,up*w+2).  `height` and `width` are
+ * x's.  up = 2 with a skip is the ("upconv", i, 1) input, up = 2 without one stage 0's, up = 1 without one the plain pad
+ * of ("upconv", i, 0) and of a Conv3x3 ("dispconv", s) head.  x, skip, out and the gradients share `dtype` (md2_dtype).
+ * up must be 1 or 2, up*h and up*w at least 2, Cx >= 1, Cs >= 0; out must have fewer than 2^31 elements
+ * (else MD2_ERR_UNSUPPORTED).  Forward is pure data movement, bit-identical to torch's chain in every dtype. ---- */
+int md2_upcat_pad(const void *x, const void *skip, void *out, int dtype, int batch, int x_channels,
+                  int skip_channels, int height, int width, int up, void *stream);
+/* The adjoint in gather form, without atomics (bitwise reproducible): each element of grad_x / grad_skip sums the
+ * padded positions that read it - its own first, then the reflected ones - and grad_x sums its up x up children in
+ * row-major order (ATen's upsample_nearest2d_backward), all in fp32 from 0.0f, rounded once to `dtype`.  grad_x and
+ * grad_skip are written (not accumulated) and may each be NULL. */
+int md2_upcat_pad_backward(const void *grad_out, void *grad_x, void *grad_skip, int dtype, int batch, int x_channels,
+                           int skip_channels, int height, int width, int up, void *stream);
+
 /* ---- monitoring path (SURVEY.md 8f-5): Trainer.compute_depth_losses, trainer.py:498-526, with
  * compute_depth_errors, layers.py:251-269.  depth = outputs[("depth",0,0)] (B,1,H,W), depth_gt (B,1,Hg,Wg);
  * metrics[7] = abs_rel, sq_rel, rmse, rmse_log, a1, a2, a3 (device floats, the order of depth_metric_names,

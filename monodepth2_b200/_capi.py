@@ -83,7 +83,7 @@ SYMBOLS = [
     "md2_scale_tensors", "md2_scale_tensors_typed", "md2_dispconv_sigmoid", "md2_dispconv_sigmoid_backward",
     "md2_dispconv_sigmoid_typed", "md2_dispconv_sigmoid_backward_typed",
     "md2_resize_plan_create", "md2_resize_plan_destroy", "md2_resize_scratch_bytes", "md2_resize_lanczos_u8",
-    "md2_color_jitter_u8",
+    "md2_color_jitter_u8", "md2_upcat_pad", "md2_upcat_pad_backward",
 ]
 
 _lib = None
@@ -119,6 +119,8 @@ def load_library(path: str = None) -> C.CDLL:
                                             C.POINTER(C.c_longlong), C.c_void_p, C.c_void_p]
     lib.md2_dispconv_sigmoid_typed.argtypes = [C.c_void_p] * 4 + [C.c_int] * 5 + [C.c_void_p]
     lib.md2_dispconv_sigmoid_backward_typed.argtypes = [C.c_void_p] * 7 + [C.c_int] * 5 + [C.c_void_p]
+    lib.md2_upcat_pad.argtypes = [C.c_void_p] * 3 + [C.c_int] * 7 + [C.c_void_p]
+    lib.md2_upcat_pad_backward.argtypes = [C.c_void_p] * 3 + [C.c_int] * 7 + [C.c_void_p]
     lib.md2_depth_metrics_scratch_bytes.argtypes = [C.c_int, C.c_int, C.c_int, C.POINTER(C.c_size_t)]
     lib.md2_depth_metrics.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_size_t] + [C.c_int] * 9 + [C.c_void_p]
     lib.md2_resize_plan_destroy.restype = None

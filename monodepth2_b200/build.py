@@ -14,7 +14,8 @@ LIB_DIR = os.path.join(HERE, "lib")
 # development knobs: MD2_LIB_NAME / MD2_NVCC_DEFS build an experimental variant next to the product library
 LIB = os.path.join(LIB_DIR, os.environ.get("MD2_LIB_NAME", "libmd2loss.so"))
 EXTRA_DEFS = os.environ.get("MD2_NVCC_DEFS", "").split()
-SOURCES = ["md2_kernels.cu", "md2_ops.cu", "md2_capi.cu", "md2_pyramid.cu", "md2_head.cu", "md2_monitor.cu"]
+SOURCES = ["md2_kernels.cu", "md2_ops.cu", "md2_capi.cu", "md2_pyramid.cu", "md2_head.cu", "md2_monitor.cu",
+           "md2_decoder.cu"]
 HEADERS = ["md2_core.cuh", "md2_pack2.cuh", "md2_roles.cuh", "md2_plan.h", os.path.join("..", "..", "include", "md2_loss.h")]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17",
               "--use_fast_math=false", "-Xcompiler", "-fPIC", "-Xptxas", "-v"]

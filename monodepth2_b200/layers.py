@@ -15,6 +15,7 @@ unfused call graph working on the same kernels' arithmetic.
 from __future__ import annotations
 
 import ctypes as C
+import types
 
 import torch
 import torch.nn as nn
@@ -25,7 +26,8 @@ from . import _capi
 __all__ = ["disp_to_depth", "transformation_from_parameters", "get_translation_matrix",
            "rot_from_axisangle", "BackprojectDepth", "Project3D", "SSIM", "get_smooth_loss",
            "grid_sample_border", "ConvBlock", "Conv3x3", "upsample", "compute_depth_errors",
-           "DispConvSigmoid", "fuse_disp_heads", "depth_metrics", "DEPTH_METRIC_NAMES"]
+           "DispConvSigmoid", "fuse_disp_heads", "upcat_pad", "fuse_decoder_stages", "depth_metrics",
+           "DEPTH_METRIC_NAMES"]
 
 
 def _lib():
@@ -388,6 +390,134 @@ def fuse_disp_heads(depth_decoder):
             if m is mod:
                 depth_decoder.decoder[i] = head
     depth_decoder.sigmoid = nn.Identity()
+    return depth_decoder
+
+
+class _UpcatPad(torch.autograd.Function):
+    """ReflectionPad2d(1)(cat([nearest_up(x, up), skip], 1)) in one pass (md2_upcat_pad), gather-form backward
+    without atomics (md2_upcat_pad_backward).  ``x`` and ``skip`` share one dtype here (``upcat_pad`` promotes)."""
+
+    @staticmethod
+    def forward(ctx, x, skip, up):
+        x = x.contiguous()
+        B, Cx, h, w = x.shape
+        Cs = 0
+        if skip is not None:
+            skip = skip.contiguous()
+            if skip.dim() != 4 or skip.shape[0] != B or tuple(skip.shape[2:]) != (up * h, up * w):
+                raise RuntimeError("upcat_pad: skip %s does not fit x %s up-sampled %dx"
+                                   % (tuple(skip.shape), tuple(x.shape), up))
+            Cs = skip.shape[1]
+        out = torch.empty((B, Cx + Cs, up * h + 2, up * w + 2), dtype=x.dtype, device=x.device)
+        ctx.dims = (_HEAD_DTYPES[x.dtype], B, Cx, Cs, h, w, up)
+        _call("md2_upcat_pad", x.device, _p(x), _p(skip), _p(out), *ctx.dims, _stream(x))
+        return out
+
+    @staticmethod
+    @torch.autograd.function.once_differentiable
+    def backward(ctx, g):
+        dt, B, Cx, Cs, h, w, up = ctx.dims
+        g = g.contiguous()
+        gx = torch.empty((B, Cx, h, w), dtype=g.dtype, device=g.device) if ctx.needs_input_grad[0] else None
+        gs = (torch.empty((B, Cs, up * h, up * w), dtype=g.dtype, device=g.device)
+              if Cs and ctx.needs_input_grad[1] else None)
+        if gx is not None or gs is not None:
+            _call("md2_upcat_pad_backward", g.device, _p(g), _p(gx), _p(gs), *ctx.dims, _stream(g))
+        return gx, gs, None
+
+
+def upcat_pad(x, skip=None, up=2):
+    """``F.pad(torch.cat([upsample(x), skip], 1), (1, 1, 1, 1), mode="reflect")`` - the input of a decoder ConvBlock
+    (networks/depth_decoder.py:48-65) - in one pass; ``up=1`` without a skip is the plain reflection pad of Conv3x3
+    (layers.py:119-136).  ``x`` (B,Cx,h,w) and ``skip`` (B,Cs,up*h,up*w) are CUDA float32, bfloat16 or float16; the
+    forward is bit-identical to torch's chain.  A skip of another dtype is promoted as ``torch.cat`` does (the narrower
+    tensor is widened with ``.to()``); each gradient comes back in its input's dtype, summed in float32 without atomics
+    and rounded once, so the backward is reproducible under ``torch.use_deterministic_algorithms(True)``."""
+    tensors = [(x, "x")] + ([(skip, "skip")] if skip is not None else [])
+    for t, name in tensors:
+        if not isinstance(t, torch.Tensor) or not t.is_cuda:
+            raise RuntimeError("upcat_pad: %s must be a CUDA tensor (monodepth2_b200.layers has no CPU path)" % name)
+        if t.dtype not in _HEAD_DTYPES:
+            raise RuntimeError("upcat_pad: %s must be float32, bfloat16 or float16, got %s" % (name, t.dtype))
+        if t.dim() != 4:
+            raise RuntimeError("upcat_pad: %s must be 4-D (B,C,H,W), got %s" % (name, tuple(t.shape)))
+    up = int(up)
+    if up not in (1, 2):
+        raise RuntimeError("upcat_pad: up must be 1 or 2, got %d" % up)
+    if skip is not None and skip.dtype != x.dtype:
+        dt = torch.promote_types(x.dtype, skip.dtype)
+        x, skip = x.to(dt), skip.to(dt)
+    return _UpcatPad.apply(x, skip, up)
+
+
+def _decoder_block(mod, key):
+    """The padding-free conv and the nonlinearity of a reference ConvBlock (layers.py:106-118) with a
+    reflection-padded Conv3x3 (layers.py:121-136); RuntimeError on anything else."""
+    conv3 = getattr(mod, "conv", None)
+    if not (isinstance(getattr(mod, "nonlin", None), nn.Module) and _is_reflect_conv3x3(conv3)):
+        raise RuntimeError("fuse_decoder_stages: convs[%r] is not a ConvBlock with a reflection-padded Conv3x3: %s"
+                           % (key, type(mod).__name__))
+    return conv3.conv, mod.nonlin
+
+
+def _is_reflect_conv3x3(m):
+    conv = getattr(m, "conv", None)
+    return (isinstance(getattr(m, "pad", None), nn.ReflectionPad2d) and tuple(m.pad.padding) == (1, 1, 1, 1)
+            and isinstance(conv, nn.Conv2d) and tuple(conv.kernel_size) == (3, 3) and tuple(conv.padding) == (0, 0)
+            and tuple(conv.stride) == (1, 1) and tuple(conv.dilation) == (1, 1) and conv.groups == 1)
+
+
+def _check_head(mod, key):
+    if not (isinstance(mod, DispConvSigmoid) or _is_reflect_conv3x3(mod)):
+        raise RuntimeError("fuse_decoder_stages: convs[%r] is neither a DispConvSigmoid nor a reflection-padded "
+                           "Conv3x3: %s" % (key, type(mod).__name__))
+
+
+def _fused_decoder_forward(self, input_features):
+    """DepthDecoder.forward (networks/depth_decoder.py:48-65) with every pad / upsample / cat done by upcat_pad."""
+    self.outputs = {}
+    x = input_features[-1]
+    for i in range(4, -1, -1):
+        conv, nonlin = _decoder_block(self.convs[("upconv", i, 0)], ("upconv", i, 0))
+        x = nonlin(conv(upcat_pad(x, up=1)))
+        skip = input_features[i - 1] if self.use_skips and i > 0 else None
+        conv, nonlin = _decoder_block(self.convs[("upconv", i, 1)], ("upconv", i, 1))
+        x = nonlin(conv(upcat_pad(x, skip, up=2)))
+        if i in self.scales:
+            head = self.convs[("dispconv", i)]
+            _check_head(head, ("dispconv", i))
+            y = head(x) if isinstance(head, DispConvSigmoid) else head.conv(upcat_pad(x, up=1))
+            self.outputs[("disp", i)] = self.sigmoid(y)
+    return self.outputs
+
+
+def fuse_decoder_stages(depth_decoder):
+    """Run every ConvBlock input of a reference DepthDecoder (networks/depth_decoder.py:17-65) through ``upcat_pad``:
+    the forward installed on ``depth_decoder`` keeps the reference's dataflow (``use_skips``, ``scales``,
+    ``num_output_channels``; it sets and returns ``self.outputs``) but runs each ConvBlock as
+    ``nonlin(conv.conv(upcat_pad(...)))`` - one pass instead of upsample + torch.cat + ReflectionPad2d, and a backward
+    without atomics.  A head fused by ``fuse_disp_heads`` is called as it is; a plain Conv3x3 head runs as
+    ``conv.conv(upcat_pad(x, up=1))``.  Either fuse call may come first.  No module or Parameter is replaced, so
+    ``state_dict`` keys and values are unchanged.  RuntimeError on a structure this does not recognise (no
+    ``convs[("upconv", i, j)]``, a zero-padded Conv3x3).  Returns the decoder."""
+    convs = getattr(depth_decoder, "convs", None)
+    if convs is None or not hasattr(convs, "items"):
+        raise RuntimeError("fuse_decoder_stages: %s has no convs dict of a reference DepthDecoder"
+                           % type(depth_decoder).__name__)
+    for i in range(4, -1, -1):
+        for j in (0, 1):
+            if ("upconv", i, j) not in convs:
+                raise RuntimeError("fuse_decoder_stages: %s has no convs[('upconv', %d, %d)]"
+                                   % (type(depth_decoder).__name__, i, j))
+            _decoder_block(convs[("upconv", i, j)], ("upconv", i, j))
+    for s in getattr(depth_decoder, "scales", ()):
+        if ("dispconv", s) not in convs:
+            raise RuntimeError("fuse_decoder_stages: scale %r has no convs[('dispconv', %r)]" % (s, s))
+        _check_head(convs[("dispconv", s)], ("dispconv", s))
+    for attr in ("use_skips", "scales", "sigmoid"):
+        if not hasattr(depth_decoder, attr):
+            raise RuntimeError("fuse_decoder_stages: %s has no %r attribute" % (type(depth_decoder).__name__, attr))
+    depth_decoder.forward = types.MethodType(_fused_decoder_forward, depth_decoder)
     return depth_decoder
 
 
