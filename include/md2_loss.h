@@ -153,7 +153,7 @@ int md2_view_synthesis_loss(const md2_problem *p, const md2_tensors *t,
                             void *workspace, size_t workspace_bytes, void *stream);
 
 /* Measurement hook (bench.py roofline leg): when enabled, every md2_view_synthesis_loss call
- * records CUDA events on its stream around the dominant kernel (md2_march);
+ * records CUDA events on its stream around the dominant kernel (md2_march_roles);
  * md2_profile_march_ms waits for the last call's pair and returns its duration. */
 int md2_profile_enable(int on);
 int md2_profile_march_ms(float *ms);

@@ -32,28 +32,17 @@
 #define MD2_LD4(p) __ldg(reinterpret_cast<const float4*>(p))
 // streaming loads (read once per job: target row, disparity, identity loss, noise): do not allocate in
 // L1, which is kept for the data-dependent gathers
-#ifndef MD2_STREAM_ALLOC
 #define MD2_LDS1(p) md2::ld_stream(p)
 #define MD2_LDS4(p) md2::ld_stream4(p)
-#else
-#define MD2_LDS1(p) __ldg(p)
-#define MD2_LDS4(p) __ldg(reinterpret_cast<const float4*>(p))
-#endif
 #define MD2_FMUL(a, b) __fmul_rn(a, b)
 #define MD2_FADD(a, b) __fadd_rn(a, b)
 #define MD2_RCP(a) md2::rcp_nr(a)
 // the SSIM ratio n/d tolerates the 1-ulp MUFU.RCP result (loss parity budget 1e-5); the depth and
 // projection reciprocals keep the Newton step because they decide bilinear cells
-#ifdef MD2_SSIM_RCP_EXACT
-#define MD2_RCP_SSIM(a) md2::rcp_nr(a)
-#else
 #define MD2_RCP_SSIM(a) md2::rcp_approx(a)
-#endif
 #define MD2_DIV(a, b) __fdiv_rn(a, b)
 #define MD2_FLOORF(a) floorf(a)
-#define MD2_PREFETCH_L1(p) asm volatile("prefetch.global.L1 [%0];" ::"l"(p))
 #else
-#define MD2_PREFETCH_L1(p) ((void)(p))
 #define MD2_LD(p) (*(p))
 #define MD2_LD4(p) (*reinterpret_cast<const md2::F4*>(p))
 #define MD2_LDS1(p) (*(p))
@@ -100,13 +89,6 @@ __device__ __forceinline__ float rcp_nr(float a) {
 #endif
 
 #if defined(__CUDACC__)
-// 16-byte asynchronous copy global -> shared (LDGSTS); tracked by the async-group counters, not by the scoreboard
-__device__ __forceinline__ void cp_async16(void* smem_dst, const void* gmem_src) {
-  asm volatile("cp.async.ca.shared.global [%0], [%1], 16;" ::"r"((unsigned)__cvta_generic_to_shared(smem_dst)), "l"(gmem_src) : "memory");
-}
-__device__ __forceinline__ void cp_async_commit() { asm volatile("cp.async.commit_group;" ::: "memory"); }
-template <int N>
-__device__ __forceinline__ void cp_async_wait() { asm volatile("cp.async.wait_group %0;" ::"n"(N) : "memory"); }
 // mbarrier + TMA bulk copy (cp.async.bulk, UBLKCP in SASS): global -> shared, completion by transaction bytes
 __device__ __forceinline__ unsigned smem_addr(const void* p) { return (unsigned)__cvta_generic_to_shared(p); }
 __device__ __forceinline__ void mbar_init(unsigned long long* bar, unsigned count) {
@@ -415,11 +397,7 @@ struct Cfg {
   static constexpr bool PAIRED = false;
   // Backward rolling state (two rows of 9*NSRC box sums): registers for up to two sources, a
   // thread-private shared-memory ring beyond that (3 sources would spill ~0.5 KB per thread).
-#ifdef MD2_BSMEM_ALL
-  static constexpr bool BSMEM = GRAD_;
-#else
   static constexpr bool BSMEM = GRAD_ && (NSRC_ >= 3);
-#endif
   // Control-flow shape of stages B/C: with 3 sources the branch-free form (every lane computes, results
   // masked) is 7 % faster, with 1-2 sources the divergent form is 3 % faster (measured, r01 log).
   static constexpr bool STRAIGHT = (NSRC_ >= 3);
@@ -473,8 +451,7 @@ MD2_HD int reflect_clamp(int i, int n) {
 }
 
 // ------------------------------------------------------------------ lane state
-// What stage_a_issue hands to stage_a_finish: the gather of one row in flight.  A separate struct so that a
-// caller can keep two rows in flight (role A of the role-specialised kernel).
+// What stage_a_issue hands to stage_a_finish: the gather of one row in flight.
 template <class C>
 struct Flight {
   F4 tap[C::NSRC][4];                           // nw, ne, sw, se texels
@@ -713,10 +690,8 @@ MD2_HD void pmask_backward(Lane<C>& L, const Params& P, const WarpJob& J, const 
 // TG_DIRECT: the target texel of row t is loaded here, straight into the slot stage_a_finish reads (it is not
 // needed before), instead of being prefetched one step ahead and moved: a move placed after the gather issue
 // waits on the gather's scoreboard (role kernel, measured: 10 % of all stall samples on that one MOV)
-// ASYNC (CUDA only): the taps are copied by cp.async (LDGSTS) into `tapdst` ([source][tap][lane] 16-byte fields of
-// shared memory) instead of being loaded into F.tap; the caller commits / waits for the group.
-template <class C, bool WITH_ID = true, int ROW_STEP = 1, bool TG_DIRECT = false, bool ASYNC = false>
-MD2_HD void stage_a_issue(Lane<C>& L, Flight<C>& F, const Params& P, const WarpJob& J, int t, F4* tapdst = nullptr) {
+template <class C, bool WITH_ID = true, int ROW_STEP = 1, bool TG_DIRECT = false>
+MD2_HD void stage_a_issue(Lane<C>& L, Flight<C>& F, const Params& P, const WarpJob& J, int t) {
   const int tr = reflect_clamp(t, J.H);
   MD2_CHK(tr * J.W + L.xi, J.plane);
   if (TG_DIRECT) {
@@ -766,36 +741,12 @@ MD2_HD void stage_a_issue(Lane<C>& L, Flight<C>& F, const Params& P, const WarpJ
     });
     const int dx1 = (x0 + 1 < J.W) ? 4 : 0;                 // texel step to the east tap
     const int dy1 = (y0 + 1 < J.H) ? J.W * 4 : 0;           // texel step to the south tap
-#if defined(MD2_KO_GATHER) && MD2_KO_GATHER == 1
-    // timing knock-out (results invalid): coalesced taps at the lane's own pixel, address still data-dependent
-    const float* t00 = J.src4[f] + 4 * (tr * J.W + L.xi + (x0 >> 30) + (y0 >> 30));
-#else
     const float* t00 = J.src4[f] + 4 * (y0 * J.W + x0);
-#endif
-#if defined(MD2_KO_GATHER) && MD2_KO_GATHER == 2
-    // timing knock-out (results invalid): no memory access at all for the taps
-    F.tap[f][0] = make_f4(ixc * 1e-3f, iyc * 1e-3f, u * 1e-3f, 0.f);
-    F.tap[f][1] = make_f4(iyc * 1e-3f, u * 1e-3f, ixc * 1e-3f, (float)(dx1 + dy1));
-    F.tap[f][2] = make_f4(v * 1e-3f, ixc * 2e-3f, iyc * 1e-3f, 0.f);
-    F.tap[f][3] = make_f4(iyc * 2e-3f, v * 1e-3f, u * 2e-3f, 0.f);
-    (void)t00;
-#else
     MD2_CHK(y0 * J.W + x0, J.plane); MD2_CHK(y0 * J.W + x0 + (dx1 + dy1) / 4, J.plane);
-#if defined(__CUDA_ARCH__)
-    if (ASYNC) {
-      cp_async16(tapdst + (f * 4 + 0) * kLanes, t00);
-      cp_async16(tapdst + (f * 4 + 1) * kLanes, t00 + dx1);
-      cp_async16(tapdst + (f * 4 + 2) * kLanes, t00 + dy1);
-      cp_async16(tapdst + (f * 4 + 3) * kLanes, t00 + dy1 + dx1);
-    } else
-#endif
-    {
-      F.tap[f][0] = MD2_LD4(t00);
-      F.tap[f][1] = MD2_LD4(t00 + dx1);
-      F.tap[f][2] = MD2_LD4(t00 + dy1);
-      F.tap[f][3] = MD2_LD4(t00 + dy1 + dx1);
-    }
-#endif
+    F.tap[f][0] = MD2_LD4(t00);
+    F.tap[f][1] = MD2_LD4(t00 + dx1);
+    F.tap[f][2] = MD2_LD4(t00 + dy1);
+    F.tap[f][3] = MD2_LD4(t00 + dy1 + dx1);
     F.cu[f] = u; F.cv[f] = v;
     F.cwx[f] = ixc - fx0; F.cwy[f] = iyc - fy0;
     F.cgx[f] = mx ? P.sx * inv : 0.0f;
@@ -805,7 +756,7 @@ MD2_HD void stage_a_issue(Lane<C>& L, Flight<C>& F, const Params& P, const WarpJ
 
 template <class C, bool WITH_ID = true, int ROW_STEP = 1, bool TG_DIRECT = false>
 MD2_HD void stage_a_issue(Lane<C>& L, const Params& P, const WarpJob& J, int t) {
-  stage_a_issue<C, WITH_ID, ROW_STEP, TG_DIRECT, false>(L, L.fl, P, J, t);
+  stage_a_issue<C, WITH_ID, ROW_STEP, TG_DIRECT>(L, L.fl, P, J, t);
 }
 
 // stage_a_finish: the taps have arrived; interpolate pred and its derivatives, export pr/tg for

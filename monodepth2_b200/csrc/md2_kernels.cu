@@ -6,14 +6,13 @@
 //   2. md2_disp_mean       per-sample mean of disp_s            (trainer.py:486)
 //   3. md2_identity        scale-independent identity losses    (trainer.py:432-439)
 //   4. md2_smooth          edge-aware smoothness, fwd + numerator gradient (layers.py:202-215)
-//   5. md2_march           fused warp + photometric loss + min/automask + adjoint, all scales
+//   5. md2_march_roles     fused warp + photometric loss + min/automask + adjoint, all scales
 //   6. md2_final           up-sampling adjoint + smoothness adjoint -> grad_disp_s, losses, grad_T
 //
-// md2_march is the hot kernel.  One warp owns a band of 28 columns and marches down a
-// segment of rows; lane l holds column x0-2+l.  Horizontal neighbours are exchanged with
-// warp shuffles, vertical neighbours live in registers (rolling 3-row sums), the values the
-// adjoint needs two rows later sit in a thread-private shared-memory ring.  No block-level
-// synchronisation, no tensor cores (the path is gather/stream work, BASELINE.json).
+// md2_march_roles (md2_roles.cuh) is the hot kernel.  One CTA owns a band of 28 columns and marches
+// down a segment of rows; lane l of each warp holds column x0-2+l, and the warps of the CTA split the
+// stages of a row between them (see md2_roles.cuh).  No tensor cores (the path is gather/stream work,
+// BASELINE.json).
 #include <cuda.h>
 #include <cuda_bf16.h>
 #include <cuda_fp16.h>
@@ -31,10 +30,7 @@
 
 namespace md2 {
 
-#ifndef MD2_WARPS_PER_CTA
-#define MD2_WARPS_PER_CTA 4
-#endif
-constexpr int kWarpsPerCta = MD2_WARPS_PER_CTA;
+constexpr int kWarpsPerCta = 4;          // identity pass (register-marching form): one job per warp
 constexpr int kThreads = kWarpsPerCta * 32;
 constexpr unsigned kFull = 0xffffffffu;
 
@@ -302,10 +298,8 @@ __global__ void __launch_bounds__(kThreads) md2_identity2(Params P) {
 // its left / right neighbours from the tile (no warp halo, no shuffles, all 32 lanes productive).  Four CTAs per
 // SM (4 x 48 KB of tiles) overlap the loads of some CTAs with the arithmetic of the others.  Used for two sources when the
 // row pitch is a multiple of 16 bytes; otherwise md2_identity / md2_identity2 run.
-#ifndef MD2_TMA_ROWS
-#define MD2_TMA_ROWS 8     // measured (whole step, 640x192 x 12): 8 rows 0.486 ms, 12 rows 0.487 ms, 16 rows 0.491 ms
-#endif
-constexpr int kTmaCols = 128, kTmaRows = MD2_TMA_ROWS;        // pixels a CTA owns
+// kTmaRows measured (whole step, 640x192 x 12): 8 rows 0.486 ms, 12 rows 0.487 ms, 16 rows 0.491 ms
+constexpr int kTmaCols = 128, kTmaRows = 8;                   // pixels a CTA owns
 constexpr int kTmaPadX = 4;      // the box starts 4 columns left of the tile: TMA needs a 16-byte aligned inner start
 constexpr int kTmaBoxW = kTmaCols + 2 * kTmaPadX, kTmaBoxH = kTmaRows + 2;   // (x0 - 1 faults with "illegal instruction")
 constexpr int kTmaImgFloats = ((3 * kTmaBoxH * kTmaBoxW * 4 + 127) / 128) * 32;   // one image's tile, 128-byte multiple
@@ -459,10 +453,7 @@ static bool make_image_map(CUtensorMap* m, const float* base, int B, int H, int 
 // down: the current row lives in registers, the next row is loaded once, so every edge is evaluated ONCE (its
 // weight exp(-|dI|) and sign serve both of its end points: right neighbour by shuffle, upper neighbour from
 // the previous step) instead of once per end point.  Same per-edge arithmetic as smooth_pixel (md2_core.cuh).
-#ifndef MD2_SMOOTH_ROWS
-#define MD2_SMOOTH_ROWS 16
-#endif
-constexpr int kSmoothRows = MD2_SMOOTH_ROWS;
+constexpr int kSmoothRows = 16;
 constexpr int kSmoothWarps = 4;
 __host__ __device__ inline int smooth_bands(int Ws) { return (Ws + 31) / 32; }
 __host__ __device__ inline int smooth_segs(int Hs) { return (Hs + kSmoothRows - 1) / kSmoothRows; }
@@ -600,204 +591,16 @@ __global__ void md2_smooth_scalars(Params P) {
   P.smsc[2 * i + 1] = dterm;
 }
 
-// ------------------------------------------------------------------ 5. the marching kernel
-#ifdef MD2_KO_SHFL   // timing knock-out (results invalid): no neighbour exchange
-#define MD2_SHUP(v) (v)
-#define MD2_SHDN(v) (v)
-#else
-#define MD2_SHUP(v) __shfl_up_sync(kFull, v, 1)
-#define MD2_SHDN(v) __shfl_down_sync(kFull, v, 1)
-#endif
-template <class C>
-__device__ __forceinline__ void exchange_and_stage_c(Lane<C>& L, const Params& P, const WarpJob& J, int t, int lane,
-                                                     const Stash& st) {
-  Xchg2<C> l2, r2;
-  l2.tag = MD2_SHUP(L.tag);
-  r2.tag = MD2_SHDN(L.tag);
-#pragma unroll
-  for (int n = 0; n < C::NCS; ++n)
-#pragma unroll
-    for (int k = 0; k < 9; ++k) {
-      l2.coef[n][k] = C::NOSSIM ? 0.f : MD2_SHUP(L.coef[n][k]);
-      r2.coef[n][k] = C::NOSSIM ? 0.f : MD2_SHDN(L.coef[n][k]);
-    }
-  stage_c(L, P, J, t, lane, l2, r2, st);
-}
-
-#define MD2_PRAGMA_(x) _Pragma(#x)
-#define MD2_PRAGMA(x) MD2_PRAGMA_(x)
-#ifdef MD2_UNROLL
-#define MD2_LOOP_UNROLL MD2_PRAGMA(unroll MD2_UNROLL)
-#else
-#define MD2_LOOP_UNROLL MD2_PRAGMA(unroll 1)
-#endif
-#if defined(MD2_MIN_CTAS)
-#define MD2_MARCH_BOUNDS __launch_bounds__(kThreads, MD2_MIN_CTAS)
-#else
-#define MD2_MARCH_BOUNDS __launch_bounds__(kThreads)
-#endif
-template <class C>
-__global__ void MD2_MARCH_BOUNDS md2_march(Params P) {
-  extern __shared__ float4 smem[];
-  const int lane = threadIdx.x & 31;
-  // warp index through a shuffle: lets the compiler treat everything derived from the job as
-  // warp-uniform (uniform registers / uniform datapath for the address arithmetic)
-  const int warp = __shfl_sync(kFull, (int)(threadIdx.x >> 5), 0);
-  const int job = blockIdx.x * kWarpsPerCta + warp;
-  // Job order: sample-major, then row segment, then scale, then band.  The four scales of one
-  // image region read the same target / source rows, so running them close together in time keeps
-  // those rows in L1/L2 (scale-major order streamed every image four times).
-  const int per_seg = P.S * P.nband;
-  const int per_b = P.nseg * per_seg;
-  if (job >= per_b * P.B) return;
-  const int jb = P.B - 1 - job / per_b;     // last sample first: the identity pass wrote it most recently (L2)
-  const int r = job - (job / per_b) * per_b;
-  const int seg = r / per_seg;
-  const int r2 = r - seg * per_seg;
-  const int js = r2 / P.nband;
-  const int jy0 = seg * P.seg_rows;
-  const WarpJob J = make_job(P, js, jb, (r2 - js * P.nband) * kOwnCols, jy0, min(jy0 + P.seg_rows, P.H));
-
-  Stash st;
-  st.base = smem + threadIdx.x;
-  st.bring = smem + kRing * C::STASH4 * kThreads + threadIdx.x;
-  st.stride = kThreads;
-  st.tbar = nullptr; st.t0 = 0;
-  bring_reset<C>(st);
-
-  Lane<C> L;
-  lane_init(L, P, J, lane);
-  MD2_LOOP_UNROLL
-  // Software-pipelined row loop: the gather of row t is issued first, the adjoint of the
-  // previous step (stage C, independent of row t) runs while it is in flight, then row t is
-  // interpolated and its window row evaluated (stage B).
-  for (int t = J.y0 - 2; t <= J.y1 + 1; ++t) {
-    stage_a_issue(L, P, J, t);
-    if (C::GRAD && t > J.y0 - 2) exchange_and_stage_c(L, P, J, t - 1, lane, st);
-    stage_a_finish(L, P, J, t, st);
-    Xchg1<C> l1, r1;
-#pragma unroll
-    for (int c = 0; c < 3; ++c) {
-      l1.tg[c] = MD2_SHUP(L.tg[c]);
-      r1.tg[c] = MD2_SHDN(L.tg[c]);
-#pragma unroll
-      for (int f = 0; f < C::NSRC; ++f) {
-        l1.pr[f][c] = MD2_SHUP(L.pr[f][c]);
-        r1.pr[f][c] = MD2_SHDN(L.pr[f][c]);
-      }
-    }
-    stage_b(L, P, J, t, lane, l1, r1);
-  }
-  if (C::GRAD) exchange_and_stage_c(L, P, J, J.y1 + 1, lane, st);
-  const float ls = warp_sum(L.loss);
-  if (lane == 0) atomicAdd(&P.acc[acc_photo(J.s)], (double)ls);
-  if (C::GRAD) {
-#pragma unroll
-    for (int f = 0; f < C::NSRC; ++f) {
-      if (!P.pose_grad[f]) continue;
-      float dP[12];
-      lane_dP(L, P, J, f, dP);
-#pragma unroll
-      for (int k = 0; k < 12; ++k) {
-        const float v = warp_sum(dP[k]);
-        if (lane == 0) atomicAdd(&P.acc[acc_dP(P, J.ps, J.b, f, k)], (double)v);
-      }
-    }
-  }
-}
-
-
-// Packed-fp32 form of md2_march for two sources (md2_pack2.cuh): same decomposition, same pipeline.
-template <class C>
-__device__ __forceinline__ void exchange_and_stage_c2(Lane2<C>& L, const Params& P, const WarpJob& J, int t, int lane,
-                                                      const Stash& st) {
-  Xchg2P<C> l2, r2;
-  l2.tag = MD2_SHUP(L.tag);
-  r2.tag = MD2_SHDN(L.tag);
-#pragma unroll
-  for (int i = 0; i < 3; ++i) {
-    l2.cf[i] = C::NOSSIM ? bc(0.f) : p2(MD2_SHUP(L.cf[i].x), MD2_SHUP(L.cf[i].y));
-    r2.cf[i] = C::NOSSIM ? bc(0.f) : p2(MD2_SHDN(L.cf[i].x), MD2_SHDN(L.cf[i].y));
-    l2.cfb[i] = C::NOSSIM ? 0.f : MD2_SHUP(L.cfb[i]);
-    r2.cfb[i] = C::NOSSIM ? 0.f : MD2_SHDN(L.cfb[i]);
-  }
-  stage_c2(L, P, J, t, lane, l2, r2, st);
-}
-
-template <class C>
-__global__ void MD2_MARCH_BOUNDS md2_march2(Params P) {
-  static_assert(C::NSRC == 2 && !C::AVG, "packed form: two sources, per-pixel minimum");
-  extern __shared__ float4 smem[];
-  const int lane = threadIdx.x & 31;
-  const int warp = __shfl_sync(kFull, (int)(threadIdx.x >> 5), 0);
-  const int job = blockIdx.x * kWarpsPerCta + warp;
-  const int per_seg = P.S * P.nband;
-  const int per_b = P.nseg * per_seg;
-  if (job >= per_b * P.B) return;
-  const int jb = P.B - 1 - job / per_b;
-  const int r = job - (job / per_b) * per_b;
-  const int seg = r / per_seg;
-  const int r2 = r - seg * per_seg;
-  const int js = r2 / P.nband;
-  const int jy0 = seg * P.seg_rows;
-  const WarpJob J = make_job(P, js, jb, (r2 - js * P.nband) * kOwnCols, jy0, min(jy0 + P.seg_rows, P.H));
-
-  Stash st;
-  st.base = smem + threadIdx.x;
-  st.bring = nullptr;
-  st.stride = kThreads;
-  st.tbar = nullptr; st.t0 = 0;
-
-  Lane2<C> L;
-  lane_init2(L, P, J, lane);
-  MD2_LOOP_UNROLL
-  for (int t = J.y0 - 2; t <= J.y1 + 1; ++t) {
-    stage_a_issue2(L, P, J, t);
-    if (C::GRAD && t > J.y0 - 2) exchange_and_stage_c2(L, P, J, t - 1, lane, st);
-    stage_a_finish2(L, P, J, t, st);
-    Xchg1P<C> l1, r1;
-    l1.tgrg = p2(MD2_SHUP(L.tgrg.x), MD2_SHUP(L.tgrg.y));
-    r1.tgrg = p2(MD2_SHDN(L.tgrg.x), MD2_SHDN(L.tgrg.y));
-    l1.tgb = MD2_SHUP(L.tgb);
-    r1.tgb = MD2_SHDN(L.tgb);
-#pragma unroll
-    for (int s = 0; s < 3; ++s) {
-      l1.pr[s] = p2(MD2_SHUP(L.pr[s].x), MD2_SHUP(L.pr[s].y));
-      r1.pr[s] = p2(MD2_SHDN(L.pr[s].x), MD2_SHDN(L.pr[s].y));
-    }
-    stage_b2(L, P, J, t, lane, l1, r1);
-  }
-  if (C::GRAD) exchange_and_stage_c2(L, P, J, J.y1 + 1, lane, st);
-  const float ls = warp_sum(L.loss);
-  if (lane == 0) atomicAdd(&P.acc[acc_photo(J.s)], (double)ls);
-  if (C::GRAD) {
-#pragma unroll
-    for (int f = 0; f < 2; ++f) {
-      if (!P.pose_grad[f]) continue;
-      float dP[12];
-      lane_dP2(L, P, J, f, dP);
-#pragma unroll
-      for (int k = 0; k < 12; ++k) {
-        const float v = warp_sum(dP[k]);
-        if (lane == 0) atomicAdd(&P.acc[acc_dP(P, J.ps, J.b, f, k)], (double)v);
-      }
-    }
-  }
-}
-
 // ------------------------------------------------------------------ 6. final
 // grad_disp_s (s >= 1) = adjoint of the bilinear up-sampling of dD_s (trainer.py:350-351) + smoothness
 // adjoint.  Separable, one pass over the fine map: a block owns kFinalFineRows fine rows x 256 fine columns;
 // pass 1, one thread per fine column (coalesced rows), folds the rows into the block's coarse rows with the
 // vertical weights and leaves them in shared memory; pass 2, one thread per coarse pixel, folds 2K columns
 // with the horizontal weights.  Every fine value is read ~1.1x (the gather form read it 4x).  Block 0 also
-// writes the losses and grad_T.  Scale 0 is finished by md2_march itself.
+// writes the losses and grad_T.  Scale 0 is finished by the marching kernel itself.
 constexpr int kFinalThreads = 256;
 // (measured at 640x192 x 12, 1 296 blocks = 1.09 waves with 16 rows: 24 rows 16.4 us, 32 rows 17.4 us, 8 rows 16.9 us, 16 rows 15.0 us)
-#ifndef MD2_FINAL_ROWS
-#define MD2_FINAL_ROWS 16
-#endif
-constexpr int kFinalFineRows = MD2_FINAL_ROWS;
+constexpr int kFinalFineRows = 16;
 
 __host__ __device__ inline int final_tiles_x(int Ws, int K) { const int t = kFinalThreads / K - 1; return (Ws + t - 1) / t; }
 __host__ __device__ inline int final_tiles_y(int Hs, int K) { const int t = kFinalFineRows / K; return (Hs + t - 1) / t; }
@@ -884,34 +687,19 @@ __global__ void __launch_bounds__(kFinalThreads) md2_final(Params P) {
 
 // ------------------------------------------------------------------ launcher
 
-// Which two-source instantiations use the packed-fp32 form (md2_pack2.cuh).  Default: forward-only calls
-// (measured faster), scalar form when gradients are wanted (measured faster).  MD2_PACK2=all / MD2_PACK2=off
-// in the environment force one form for every two-source call (A/B checks, tests/test_gpu_parity.py).
-static int pack2_mode() {
+// Whether the two-source kernels that have a packed-fp32 form (md2_pack2.cuh) use it: the marching kernel's roles A
+// and B, and the identity pass.  MD2_PACK2=off in the environment forces the scalar form for every call (A/B checks,
+// tests/test_gpu_parity.py).
+static bool pack2_on() {
 #ifdef MD2_DBG_DEVICE
-  return 0;      // the decision export lives in the scalar stage functions
-#endif
-  static const int mode = [] {
+  return false;      // the decision export lives in the scalar stage functions
+#else
+  static const bool on = [] {
     const char* e = getenv("MD2_PACK2");
-    if (e && !strcmp(e, "all")) return 2;
-    if (e && !strcmp(e, "off")) return 0;
-    return 1;
+    return !(e && !strcmp(e, "off"));
   }();
-  return mode;
-}
-static bool use_pack2(bool grad) { return pack2_mode() == 2 || (pack2_mode() == 1 && !grad); }
-
-// Which form of the marching kernel runs.  Default: the role-specialised kernel (md2_roles.cuh).
-// MD2_MARCH=warp selects the round-1 one-warp-per-band kernels (md2_march / md2_march2) for A/B checks.
-static int march_mode() {
-  static const int mode = [] {
-    const char* e = getenv("MD2_MARCH");
-    if (e && !strcmp(e, "warp")) return 0;
-    if (e && !strcmp(e, "flow")) return 2;
-    if (e && !strcmp(e, "lockstep")) return 3;
-    return 1;
-  }();
-  return mode;
+  return on;
+#endif
 }
 
 static int device_sm_count() {
@@ -931,50 +719,12 @@ static cudaError_t launch_march_roles(const Params& P0, cudaStream_t stream) {
   Params P = P0;
   P.nsm = device_sm_count();
   const int jobs = P.S * P.B * P.nseg * P.nband;
-#ifdef MD2_WITH_FLOW
-  if (march_mode() == 2) {           // MD2_MARCH=flow: free-running roles (experimental, measured 2.4x slower)
-    typedef FlowCfg<C> FC;
-    const size_t fsmem = (size_t)FC::SMEM_F4 * sizeof(float4);
-    if constexpr (C::NSRC == 2 && !C::AVG) {
-      if (pack2_mode() != 0) {
-        static cudaError_t a2 = cudaFuncSetAttribute(md2_march_flow<C, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)fsmem);
-        if (a2 != cudaSuccess) return a2;
-        md2_march_flow<C, true><<<jobs, FC::THREADS, fsmem, stream>>>(P);
-        return cudaGetLastError();
-      }
-    }
-    static cudaError_t a1 = cudaFuncSetAttribute(md2_march_flow<C, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)fsmem);
-    if (a1 != cudaSuccess) return a1;
-    md2_march_flow<C, false><<<jobs, FC::THREADS, fsmem, stream>>>(P);
-    return cudaGetLastError();
-  }
-#endif
   const size_t smem = (size_t)RC::SMEM_F4 * sizeof(float4);
-#ifdef MD2_WITH_MB
-  if constexpr (C::NSRC == 2 && !C::AVG && C::AUTOMASK && C::GRAD) {
-    // decoupled roles (mbarrier pipeline, md2_march_mb) for the packed two-source kernels with gradients;
-    // MD2_MARCH=lockstep keeps the one-barrier-per-row kernel
-    if (pack2_mode() != 0 && march_mode() == 1) {
-      typedef MbCfg<PairedOf<C>> MC;
-      const size_t msmem = (size_t)MC::SMEM_F4 * sizeof(float4);
-      static cudaError_t attrm = cudaFuncSetAttribute(md2_march_mb<C>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)msmem);
-      if (attrm != cudaSuccess) return attrm;
-      md2_march_mb<C><<<jobs, MC::THREADS, msmem, stream>>>(P);
-      return cudaGetLastError();
-    }
-  }
-#endif
   if constexpr (C::NSRC == 2 && !C::AVG && (C::AUTOMASK || !C::GRAD)) {
-    if (pack2_mode() != 0) {          // packed-fp32 roles unless MD2_PACK2=off (--disable_automasking with
+    if (pack2_on()) {                 // packed-fp32 roles unless MD2_PACK2=off (--disable_automasking with
                                       // gradients: the packed form spills 16 bytes under 128 registers, scalar fits)
       static cudaError_t attr2 = cudaFuncSetAttribute(md2_march_roles<C, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
       if (attr2 != cudaSuccess) return attr2;
-#ifdef MD2_DEV_KNOBS
-      // development knob: shared-memory carve-out in per cent of the unified L1 / shared memory (default: the driver's pick)
-      static const int carve = getenv("MD2_CARVEOUT") ? atoi(getenv("MD2_CARVEOUT")) : -1;
-      static cudaError_t attr3 = carve >= 0 ? cudaFuncSetAttribute(md2_march_roles<C, true>, cudaFuncAttributePreferredSharedMemoryCarveout, carve) : cudaSuccess;
-      if (attr3 != cudaSuccess) return attr3;
-#endif
       md2_march_roles<C, true><<<jobs, RC::THREADS, smem, stream>>>(P);
       return cudaGetLastError();
     }
@@ -985,53 +735,18 @@ static cudaError_t launch_march_roles(const Params& P0, cudaStream_t stream) {
   return cudaGetLastError();
 }
 
-template <class C>
-static cudaError_t launch_march(const Params& P, cudaStream_t stream) {
-#ifndef MD2_WITH_WARP_KERNELS
-  // the round-1 one-warp-per-band kernels (md2_march / md2_march2) are compiled only with -DMD2_WITH_WARP_KERNELS
-  // (A/B measurements); the product library holds the role-specialised kernels alone
-  return launch_march_roles<C>(P, stream);
-#else
-  if (march_mode() != 0 || C::NSRC > 3) return launch_march_roles<C>(P, stream);
-  const int jobs = P.S * P.B * P.nseg * P.nband;
-  const int grid = (jobs + kWarpsPerCta - 1) / kWarpsPerCta;
-  size_t smem = (size_t)kThreads * C::SMEM4 * sizeof(float4);
-#ifdef MD2_DEV_KNOBS
-  // development knob: pad the dynamic shared memory to lower the number of resident warps per SM
-  static const int pad = getenv("MD2_PAD_SMEM") ? atoi(getenv("MD2_PAD_SMEM")) : 0;
-  smem += (size_t)pad;
-#endif
-  if (smem > 48 * 1024) {
-    cudaError_t e = cudaFuncSetAttribute(md2_march<C>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-    if (e != cudaSuccess) return e;
-  }
-  if constexpr (C::NSRC == 2 && !C::AVG) {
-    if (use_pack2(C::GRAD)) {
-      if (smem > 48 * 1024) {
-        cudaError_t e = cudaFuncSetAttribute(md2_march2<C>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-        if (e != cudaSuccess) return e;
-      }
-      md2_march2<C><<<grid, kThreads, smem, stream>>>(P);
-      return cudaGetLastError();
-    }
-  }
-  md2_march<C><<<grid, kThreads, smem, stream>>>(P);
-  return cudaGetLastError();
-#endif
-}
-
 template <int NSRC, bool NOSSIM>
 static cudaError_t launch_march_n(const Params& P, cudaStream_t stream) {
   const int key = (P.avg ? 4 : 0) | (P.automask ? 2 : 0) | (P.want_grad ? 1 : 0);
   switch (key) {
-    case 0: return launch_march<Cfg<NSRC, false, false, false, NOSSIM>>(P, stream);
-    case 1: return launch_march<Cfg<NSRC, false, false, true, NOSSIM>>(P, stream);
-    case 2: return launch_march<Cfg<NSRC, false, true, false, NOSSIM>>(P, stream);
-    case 3: return launch_march<Cfg<NSRC, false, true, true, NOSSIM>>(P, stream);
-    case 4: return launch_march<Cfg<NSRC, true, false, false, NOSSIM>>(P, stream);
-    case 5: return launch_march<Cfg<NSRC, true, false, true, NOSSIM>>(P, stream);
-    case 6: return launch_march<Cfg<NSRC, true, true, false, NOSSIM>>(P, stream);
-    default: return launch_march<Cfg<NSRC, true, true, true, NOSSIM>>(P, stream);
+    case 0: return launch_march_roles<Cfg<NSRC, false, false, false, NOSSIM>>(P, stream);
+    case 1: return launch_march_roles<Cfg<NSRC, false, false, true, NOSSIM>>(P, stream);
+    case 2: return launch_march_roles<Cfg<NSRC, false, true, false, NOSSIM>>(P, stream);
+    case 3: return launch_march_roles<Cfg<NSRC, false, true, true, NOSSIM>>(P, stream);
+    case 4: return launch_march_roles<Cfg<NSRC, true, false, false, NOSSIM>>(P, stream);
+    case 5: return launch_march_roles<Cfg<NSRC, true, false, true, NOSSIM>>(P, stream);
+    case 6: return launch_march_roles<Cfg<NSRC, true, true, false, NOSSIM>>(P, stream);
+    default: return launch_march_roles<Cfg<NSRC, true, true, true, NOSSIM>>(P, stream);
   }
 }
 template <int NSRC>
@@ -1046,7 +761,7 @@ static void launch_identity_ns(const Params& P, int grid, cudaStream_t stream) {
     static const bool tma_on = !(getenv("MD2_IDENTITY_TMA") && atoi(getenv("MD2_IDENTITY_TMA")) == 0);
     uintptr_t bits = (uintptr_t)P.tgt;
     for (int f = 0; f < NSRC; ++f) bits |= (uintptr_t)P.src[f];
-    if (tma_on && !P.tgt8 && pack2_mode() != 0 && (bits & 15) == 0 && P.W % 4 == 0 && P.W >= kTmaBoxW && P.H >= kTmaBoxH) {
+    if (tma_on && !P.tgt8 && pack2_on() && (bits & 15) == 0 && P.W % 4 == 0 && P.W >= kTmaBoxW && P.H >= kTmaBoxH) {
       IdTensorMaps maps;
       bool ok = make_image_map(&maps.img[0], P.tgt, P.B, P.H, P.W);
       for (int f = 0; f < NSRC && ok; ++f) ok = make_image_map(&maps.img[1 + f], P.src[f], P.B, P.H, P.W);
@@ -1073,7 +788,7 @@ static void launch_identity_ns(const Params& P, int grid, cudaStream_t stream) {
     }
   }
   if constexpr (NSRC == 2) {
-    if (pack2_mode() != 0) {      // the identity pass is forward-only: packed form unless MD2_PACK2=off
+    if (pack2_on()) {      // the identity pass is forward-only: packed form unless MD2_PACK2=off
       if (P.no_ssim) md2_identity2<true><<<grid, kThreads, 0, stream>>>(P);
       else md2_identity2<false><<<grid, kThreads, 0, stream>>>(P);
       return;
@@ -1248,7 +963,7 @@ static cudaError_t launch_float_entry(const Params& P, cudaStream_t stream) {
   // ---- main stream: depth planes (role kernels), (identity + re-layout) or re-layout alone, then the marching kernel
   // (measured at 640x192 x 12: on the caller's stream in front of the identity pass the 12 us of md2_depth_up are
   // fully exposed; on the smoothness side stream they are too, that stream being as long as the identity pass)
-  const bool zup = (march_mode() != 0 || P.nsrc > 3) && P.S > P.up0;
+  const bool zup = P.S > P.up0;
   if (zup) {
     if ((e = cudaStreamWaitEvent(side->stream2, side->fork, 0)) != cudaSuccess) return e;
     dim3 grid((P.W + kDupCols - 1) / kDupCols, (P.H + kDupRows - 1) / kDupRows, P.B * (P.S - P.up0));

@@ -18,9 +18,10 @@
 // ~37 % fewer FP32 issue slots than the scalar form (static loop 1245 -> 1067 instructions).  Measured on
 // B200 (profiles/r01_optimization_log.md): the forward-only kernel (154 registers, 12 warps per SM) gets
 // 23 % faster (0.272 -> 0.209 ms), the forward+adjoint kernel sits at the 255-register cap either way and
-// is latency-bound at 8 warps per SM: 0.443 ms packed vs 0.427 ms scalar.  The library therefore uses the
-// packed form for forward-only calls (validation, trainer.py:320-339) and the scalar form when gradients
-// are wanted; MD2_PACK2=all / MD2_PACK2=off in the environment force one form (A/B tests).
+// is latency-bound at 8 warps per SM: 0.443 ms packed vs 0.427 ms scalar.  The role-specialised kernel
+// (md2_roles.cuh) runs its roles A and B in this form for two sources without --avg_reprojection (except
+// --disable_automasking with gradients), and so does the identity pass; MD2_PACK2=off in the environment
+// forces the scalar form (A/B tests).
 // Device-only (the emulator keeps the scalar form; tests/test_gpu_parity.py ties the two together).
 #pragma once
 
@@ -129,12 +130,6 @@ struct Xchg1P {
   P2 tgrg;
   float tgb;
 };
-template <class C>
-struct Xchg2P {
-  P2 cf[3];
-  float cfb[3];
-  int tag;
-};
 
 template <class C, bool WITH_TG = true>
 __device__ __forceinline__ void prefetch_row2(Lane2<C>& L, const WarpJob& J, int t) {
@@ -222,52 +217,37 @@ __device__ __forceinline__ void load_identity_row2(Lane2<C>& L, const WarpJob& J
   }
 }
 
-// UNI: the lane-invariant projection rows (qb, p4 over the two sources; 6 float2) are read from shared memory
-// (`uni`, broadcast LDS) instead of living in 12 registers, and the target texel is left to the caller (role_a2_pipe
-// keeps ONE copy for the row being interpolated instead of one per Flight record).
-// ZEXT: the depth of the row comes from shared memory (`zsrc`, written by role C one period earlier, see c_publish_z
-// in md2_roles.cuh): no disparity loads, up-sampling or reciprocal in this warp.
-template <class C, bool WITH_ID = true, int ROW_STEP = 1, bool TG_DIRECT = false, bool ASYNC = false, bool UNI = false, bool ZEXT = false>
-__device__ __forceinline__ void stage_a_issue2(Lane2<C>& L, Flight2& F, const Params& P, const WarpJob& J, int t, F4* tapdst = nullptr,
-                                               const P2* uni = nullptr, const float* zsrc = nullptr) {
+template <class C, bool WITH_ID = true, int ROW_STEP = 1, bool TG_DIRECT = false>
+__device__ __forceinline__ void stage_a_issue2(Lane2<C>& L, Flight2& F, const Params& P, const WarpJob& J, int t) {
   const int tr = reflect_clamp(t, J.H);
-  if (UNI) {
-  } else if (TG_DIRECT) {
+  if (TG_DIRECT) {
     if (J.staged) F.ctg = make_f4(0.f, 0.f, 0.f, 0.f);      // the row goes into the ring by TMA
     else F.ctg = MD2_LDS4(J.tgt4 + 4 * (tr * J.W + L.xi));
   } else F.ctg = L.ntg;
-  float z;
-  if (ZEXT) {
-    z = *zsrc;
-    if (WITH_ID) load_identity_row2(L, J, t);
+  float D = 0.f, zpre = 0.f;
+  if (C::ZUP) {
+    zpre = L.nd[0];
+  } else if (J.s == 0) {
+    D = L.nd[0];
   } else {
-    float D = 0.f, zpre = 0.f;
-    if (C::ZUP) {
-      zpre = L.nd[0];
-    } else if (J.s == 0) {
-      D = L.nd[0];
-    } else {
-      float syr = fmaf(J.rs, (float)tr + 0.5f, -0.5f);
-      syr = syr < 0.0f ? 0.0f : syr;
-      const float l1 = syr - (float)(int)syr, l0 = 1.0f - l1;
-      const float top = up_blend(L.ul0, L.nd[0], L.ul1, L.nd[1]);
-      const float bot = up_blend(L.ul0, L.nd[2], L.ul1, L.nd[3]);
-      D = up_blend(l0, top, l1, bot);
-    }
-    if (ROW_STEP > 0) prefetch_row2<C, !TG_DIRECT>(L, J, t + ROW_STEP);
-    if (WITH_ID) load_identity_row2(L, J, t);
-    z = C::ZUP ? (J.s == 0 ? depth_of_disp(P, zpre) : zpre) : depth_of_disp(P, D);
+    float syr = fmaf(J.rs, (float)tr + 0.5f, -0.5f);
+    syr = syr < 0.0f ? 0.0f : syr;
+    const float l1 = syr - (float)(int)syr, l0 = 1.0f - l1;
+    const float top = up_blend(L.ul0, L.nd[0], L.ul1, L.nd[1]);
+    const float bot = up_blend(L.ul0, L.nd[2], L.ul1, L.nd[3]);
+    D = up_blend(l0, top, l1, bot);
   }
+  if (ROW_STEP > 0) prefetch_row2<C, !TG_DIRECT>(L, J, t + ROW_STEP);
+  if (WITH_ID) load_identity_row2(L, J, t);
+  const float z = C::ZUP ? (J.s == 0 ? depth_of_disp(P, zpre) : zpre) : depth_of_disp(P, D);
   F.cz = z;
   const float yf = (float)tr;
-  const P2 qb0 = UNI ? uni[0] : L.qb[0], qb1 = UNI ? uni[1] : L.qb[1], qb2 = UNI ? uni[2] : L.qb[2];
-  const P2 p40 = UNI ? uni[3] : L.p4[0], p41 = UNI ? uni[4] : L.p4[1], p42 = UNI ? uni[5] : L.p4[2];
-  const P2 q0 = fma2(qb0, bc(yf), L.qa[0]);
-  const P2 q1 = fma2(qb1, bc(yf), L.qa[1]);
-  const P2 q2 = fma2(qb2, bc(yf), L.qa[2]);
-  const P2 c0 = fma2(bc(z), q0, p40);
-  const P2 c1 = fma2(bc(z), q1, p41);
-  const P2 c2 = fma2(bc(z), q2, p42);
+  const P2 q0 = fma2(L.qb[0], bc(yf), L.qa[0]);
+  const P2 q1 = fma2(L.qb[1], bc(yf), L.qa[1]);
+  const P2 q2 = fma2(L.qb[2], bc(yf), L.qa[2]);
+  const P2 c0 = fma2(bc(z), q0, L.p4[0]);
+  const P2 c1 = fma2(bc(z), q1, L.p4[1]);
+  const P2 c2 = fma2(bc(z), q2, L.p4[2]);
   const P2 den = add2(c2, bc(P.eps));
   const P2 r0 = p2(rcp_fast(den.x), rcp_fast(den.y));
   const P2 inv = fma2(r0, fma2(neg2(den), r0, bc(1.0f)), r0);      // Newton step of rcp_nr
@@ -290,41 +270,16 @@ __device__ __forceinline__ void stage_a_issue2(Lane2<C>& L, Flight2& F, const Pa
     const int dx1 = (x0 + 1 < J.W) ? 4 : 0;
     const int dy1 = (y0 + 1 < J.H) ? J.W * 4 : 0;
     const float* t00 = J.src4[f] + 4 * (y0 * J.W + x0);
-    if (ASYNC) {
-      cp_async16(tapdst + (f * 4 + 0) * kLanes, t00);
-      cp_async16(tapdst + (f * 4 + 1) * kLanes, t00 + dx1);
-      cp_async16(tapdst + (f * 4 + 2) * kLanes, t00 + dy1);
-      cp_async16(tapdst + (f * 4 + 3) * kLanes, t00 + dy1 + dx1);
-    } else {
-#if defined(MD2_TAP_SPLIT) && defined(__CUDA_ARCH__)
-      // 8-byte + 4-byte load per texel instead of one 16-byte load: no register is tied up by the unused 4th component
-      auto ld3 = [](const float* p) {
-        const float2 a = __ldg(reinterpret_cast<const float2*>(p));
-        return make_f4(a.x, a.y, __ldg(p + 2), 0.f);
-      };
-      F.tap[f][0] = ld3(t00);
-      F.tap[f][1] = ld3(t00 + dx1);
-      F.tap[f][2] = ld3(t00 + dy1);
-      F.tap[f][3] = ld3(t00 + dy1 + dx1);
-#else
-      F.tap[f][0] = MD2_LD4(t00);
-      F.tap[f][1] = MD2_LD4(t00 + dx1);
-      F.tap[f][2] = MD2_LD4(t00 + dy1);
-      F.tap[f][3] = MD2_LD4(t00 + dy1 + dx1);
-#endif
-    }
-#ifdef MD2_TAP_PREFETCH
-    // the next image row gathers (to first order) one source row further down: its upper taps are this row's lower
-    // taps (already in L1), its lower taps are pulled into L1 now - no destination register, no scoreboard - so that
-    // the gather issued one period later does not pay the L2 / HBM latency inside role A, the role every barrier waits for
-    MD2_PREFETCH_L1(t00 + ((y0 + MD2_TAP_PREFETCH < J.H) ? MD2_TAP_PREFETCH * J.W * 4 : dy1));
-#endif
+    F.tap[f][0] = MD2_LD4(t00);
+    F.tap[f][1] = MD2_LD4(t00 + dx1);
+    F.tap[f][2] = MD2_LD4(t00 + dy1);
+    F.tap[f][3] = MD2_LD4(t00 + dy1 + dx1);
   }
 }
 
 template <class C, bool WITH_ID = true, int ROW_STEP = 1, bool TG_DIRECT = false>
 __device__ __forceinline__ void stage_a_issue2(Lane2<C>& L, const Params& P, const WarpJob& J, int t) {
-  stage_a_issue2<C, WITH_ID, ROW_STEP, TG_DIRECT, false>(L, L.fl, P, J, t);
+  stage_a_issue2<C, WITH_ID, ROW_STEP, TG_DIRECT>(L, L.fl, P, J, t);
 }
 
 // stage_a_issue2 in two halves (Cfg::ZUP kernels): everything up to the tap addresses of row t ...
@@ -364,12 +319,12 @@ __device__ __forceinline__ void stage_a_proj2(Lane2<C>& L, Proj2& R, const Param
     R.dy1[f] = (y0 + 1 < J.H) ? J.W * 4 : 0;
   }
 }
-// ... and the gather itself (plus the target texel of bands that are not staged by TMA)
-template <class C, bool COPY = true>
+// ... and the gather itself (plus the target texel of bands that are not staged by TMA); the caller moves the rest of
+// the record into F after its next stage_a_proj2
+template <class C>
 __device__ __forceinline__ void stage_a_gather2(const Lane2<C>& L, Flight2& F, const Proj2& R, const WarpJob& J, int t) {
   if (J.staged) F.ctg = make_f4(0.f, 0.f, 0.f, 0.f);
   else F.ctg = MD2_LDS4(J.tgt4 + 4 * (reflect_clamp(t, J.H) * J.W + L.xi));
-  if (COPY) { F.cz = R.cz; F.cu = R.cu; F.cv = R.cv; F.cwx = R.cwx; F.cwy = R.cwy; F.cgx = R.cgx; F.cgy = R.cgy; }
 #pragma unroll
   for (int f = 0; f < 2; ++f) {
     const int dx1 = R.dx1[f], dy1 = R.dy1[f];
@@ -395,12 +350,6 @@ __device__ __forceinline__ void stage_a_finish2(Lane2<C>& L, const Flight2& F, c
 #pragma unroll
   for (int f = 0; f < 2; ++f) {
     const F4 nw = F.tap[f][0], ne = F.tap[f][1], sw = F.tap[f][2], se = F.tap[f][3];
-#if defined(MD2_KEEP_W) && defined(__CUDA_ARCH__)
-    // the unused 4th component of a texel load stays reserved until the load is consumed: ptxas otherwise reuses the
-    // register as scratch while the load is in flight, and the write waits for the load (measured: 1 700 of A's 8 300
-    // stall samples on one such FSEL / MOV)
-    asm volatile("" ::"f"(nw.w), "f"(ne.w), "f"(sw.w), "f"(se.w));
-#endif
     const float wx = f ? F.cwx.y : F.cwx.x, wy = f ? F.cwy.y : F.cwy.x;
     const float gxs = f ? F.cgx.y : F.cgx.x, gys = f ? F.cgy.y : F.cgy.x;
     // channels (r,g) as a pair
@@ -442,111 +391,8 @@ __device__ __forceinline__ void stage_a_finish2(Lane2<C>& L, const Params& P, co
   stage_a_finish2<C, ST, PUBLISH>(L, L.fl, P, J, t, st);
 }
 
-// ------------------------------------------------------------------ stage B (see stage_b_divergent)
-template <class C>
-__device__ __forceinline__ void stage_b2(Lane2<C>& L, const Params& P, const WarpJob& J, int t, int lane,
-                                         const Xchg1P<C>& lf, const Xchg1P<C>& rt) {
-  const int yw = t - 1;
-  P2 H0[3][3], HYrg0[2];
-  float HYb0[2];
-  HYrg0[0] = add2(add2(lf.tgrg, L.tgrg), rt.tgrg);
-  HYrg0[1] = fma2(rt.tgrg, rt.tgrg, fma2(L.tgrg, L.tgrg, mul2(lf.tgrg, lf.tgrg)));
-  HYb0[0] = lf.tgb + L.tgb + rt.tgb;
-  HYb0[1] = fmaf(rt.tgb, rt.tgb, fmaf(L.tgb, L.tgb, lf.tgb * lf.tgb));
-#pragma unroll
-  for (int s = 0; s < 3; ++s) {
-    const P2 yl = (s < 2) ? lf.tgrg : bc(lf.tgb), yc = (s < 2) ? L.tgrg : bc(L.tgb), yr = (s < 2) ? rt.tgrg : bc(rt.tgb);
-    const P2 xl = lf.pr[s], xc = L.pr[s], xr = rt.pr[s];
-    H0[s][0] = add2(add2(xl, xc), xr);
-    H0[s][1] = fma2(xr, xr, fma2(xc, xc, mul2(xl, xl)));
-    H0[s][2] = fma2(xr, yr, fma2(xc, yc, mul2(xl, yl)));
-  }
-  const bool win_ok = L.colok && (yw >= 0) && (yw < P.H) && (lane >= 1) && (lane <= kLanes - 2) &&
-                      (yw >= J.y0 - (C::GRAD ? 1 : 0)) && (yw < J.y1 + (C::GRAD ? 1 : 0));
-  const bool own_win = win_ok && (lane >= 2) && (lane < 2 + kOwnCols) && (yw >= J.y0) && (yw < J.y1);
-  int tag = -1;
-#pragma unroll
-  for (int i = 0; i < 3; ++i) { L.cf[i] = bc(0.f); L.cfb[i] = 0.f; }
-  if (win_ok) {
-    P2 V[3][3], VYrg[2];
-    float VYb[2];
-#pragma unroll
-    for (int k = 0; k < 2; ++k) { VYrg[k] = add2(L.HYrg2[k], HYrg0[k]); VYb[k] = L.HYb2[k] + HYb0[k]; }
-#pragma unroll
-    for (int s = 0; s < 3; ++s)
-#pragma unroll
-      for (int k = 0; k < 3; ++k) V[s][k] = add2(L.H2[s][k], H0[s][k]);
-    P2 S[3];
-#pragma unroll
-    for (int s = 0; s < 3; ++s) {
-      S[s] = bc(0.f);
-      if (!C::NOSSIM)
-        S[s] = ssim_window2(V[s][0], V[s][1], V[s][2], (s < 2) ? VYrg[0] : bc(VYb[0]), (s < 2) ? VYrg[1] : bc(VYb[1]), nullptr);
-    }
-    const P2 e0 = sub2(L.tgrg1, L.pr1[0]), e1 = sub2(L.tgrg1, L.pr1[1]), e2 = sub2(bc(L.tgb1), L.pr1[2]);
-    float rl[2];
-    {
-      const float ss0 = ((0.f + S[0].x) + S[0].y) + S[2].x, ss1 = ((0.f + S[1].x) + S[1].y) + S[2].y;
-      const float l10 = ((0.f + fabsf(e0.x)) + fabsf(e0.y)) + fabsf(e2.x);
-      const float l11 = ((0.f + fabsf(e1.x)) + fabsf(e1.y)) + fabsf(e2.y);
-      rl[0] = C::NOSSIM ? l10 * (1.0f / 3.0f) : fmaf(0.85f / 3.0f, ss0, (0.15f / 3.0f) * l10);
-      rl[1] = C::NOSSIM ? l11 * (1.0f / 3.0f) : fmaf(0.85f / 3.0f, ss1, (0.15f / 3.0f) * l11);
-    }
-    float best = INFINITY;
-    if (C::AUTOMASK) {
-#pragma unroll
-      for (int f = 0; f < 2; ++f) {
-        const float cand = MD2_FADD(L.idv[f], MD2_FMUL(L.nzv[f], 0.00001f));
-        if (cand < best) best = cand;
-      }
-    }
-    const bool pm = !C::AUTOMASK && J.pm;             // --predictive_mask (see pmask_apply in md2_core.cuh)
-#pragma unroll
-    for (int f = 0; f < 2; ++f) {
-      const float cand = pm ? rl[f] * L.nzv[f] : rl[f];
-      if (cand < best) { best = cand; tag = f; }
-    }
-    if (own_win) {
-      L.loss += best;
-      if (C::AUTOMASK && J.idsel) J.idsel[yw * J.W + L.xi] = (tag >= 0) ? 1.0f : 0.0f;
-      if (pm && C::GRAD && J.gpm) {
-#pragma unroll
-        for (int f = 0; f < 2; ++f) J.gpm[f * J.plane + yw * J.W + L.xi] = (tag == f) ? rl[f] * P.gscale : 0.0f;
-      }
-    }
-    if (C::GRAD && !C::NOSSIM && tag >= 0) {
-      // the winner's window sums: (r,g) pair from slot `tag`, b from that half of slot 2
-      const bool w1 = (tag == 1);
-      P2 Wrg[3];
-      float Wb[3];
-#pragma unroll
-      for (int k = 0; k < 3; ++k) { Wrg[k] = sel2(w1, V[1][k], V[0][k]); Wb[k] = w1 ? V[2][k].y : V[2][k].x; }
-      ssim_window2(Wrg[0], Wrg[1], Wrg[2], VYrg[0], VYrg[1], L.cf);
-      ssim_window(Wb[0], Wb[1], Wb[2], VYb[0], VYb[1], L.cfb);
-      if (pm) {
-        const float m = w1 ? L.nzv[1] : L.nzv[0];
-#pragma unroll
-        for (int k = 0; k < 3; ++k) { L.cf[k] = mul2(L.cf[k], bc(m)); L.cfb[k] *= m; }
-      }
-    }
-  }
-  L.tag = tag;
-  // roll the forward state
-#pragma unroll
-  for (int k = 0; k < 2; ++k) {
-    L.HYrg2[k] = add2(L.HYrg1[k], HYrg0[k]); L.HYrg1[k] = HYrg0[k];
-    L.HYb2[k] = L.HYb1[k] + HYb0[k]; L.HYb1[k] = HYb0[k];
-  }
-  L.tgrg1 = L.tgrg; L.tgb1 = L.tgb;
-#pragma unroll
-  for (int s = 0; s < 3; ++s) {
-#pragma unroll
-    for (int k = 0; k < 3; ++k) { L.H2[s][k] = add2(L.H1[s][k], H0[s][k]); L.H1[s][k] = H0[s][k]; }
-    L.pr1[s] = L.pr[s];
-  }
-}
-
-// Branch-free form of stage_b2 (MD2_B2_STRAIGHT): every lane computes the window, results are selected.
+// ------------------------------------------------------------------ stage B (see stage_b_straight)
+// Branch-free: every lane computes the window, results are selected.
 template <class C>
 __device__ __forceinline__ void stage_b2_straight(Lane2<C>& L, const Params& P, const WarpJob& J, int t, int lane,
                                          const Xchg1P<C>& lf, const Xchg1P<C>& rt) {
@@ -653,95 +499,6 @@ __device__ __forceinline__ void stage_b2_straight(Lane2<C>& L, const Params& P, 
     for (int k = 0; k < 3; ++k) { L.H2[s][k] = add2(L.H1[s][k], H0[s][k]); L.H1[s][k] = H0[s][k]; }
     L.pr1[s] = L.pr[s];
   }
-}
-
-// ------------------------------------------------------------------ stage C (see stage_c_divergent)
-template <class C, class ST>
-__device__ __forceinline__ void stage_c2(Lane2<C>& L, const Params& P, const WarpJob& J, int t, int lane,
-                                         const Xchg2P<C>& lf, const Xchg2P<C>& rt, const ST& st) {
-  const int yp = t - 2;
-  const float wl = (L.x == 1) ? 2.0f : 1.0f;
-  const float wr = (L.x == P.W - 2) ? 2.0f : 1.0f;
-  float ml[2], mc[2], mr[2];
-#pragma unroll
-  for (int f = 0; f < 2; ++f) {
-    ml[f] = (lf.tag == f) ? wl : 0.0f;
-    mc[f] = (L.tag == f) ? 1.0f : 0.0f;
-    mr[f] = (rt.tag == f) ? wr : 0.0f;
-  }
-  P2 B0rg[2][3], B0b[3];
-#pragma unroll
-  for (int i = 0; i < 3; ++i) {
-#pragma unroll
-    for (int f = 0; f < 2; ++f)
-      B0rg[f][i] = fma2(bc(ml[f]), lf.cf[i], fma2(bc(mr[f]), rt.cf[i], mul2(bc(mc[f]), L.cf[i])));
-    B0b[i] = fma2(p2(ml[0], ml[1]), bc(lf.cfb[i]), fma2(p2(mr[0], mr[1]), bc(rt.cfb[i]), mul2(p2(mc[0], mc[1]), bc(L.cfb[i]))));
-  }
-  const bool own = L.colok && (lane >= 2) && (lane < 2 + kOwnCols) && (yp >= J.y0) && (yp < J.y1);
-  if (own) {
-    const P2 (&B1rg)[2][3] = L.B1rg, (&B2rg)[2][3] = L.B2rg;
-    const P2 (&B1b)[3] = L.B1b, (&B2b)[3] = L.B2b;
-    const float wu = (yp == 1) ? 2.0f : 1.0f;
-    const float wd = (yp == P.H - 2) ? 2.0f : 1.0f;
-    const int slot = st.slot(yp);
-    const F4 s0 = st.at(slot, 0, C::STASH4);
-    const P2 tgrg = p2(s0.x, s0.y);
-    const float tgb = s0.z, z = st.at(slot, 3, C::STASH4).w;
-    const float yf = (float)yp;
-    // channel b box adjoint, over the two sources
-    const P2 Ab = fma2(bc(wu), B2b[0], fma2(bc(wd), B0b[0], B1b[0]));
-    const P2 Bb = fma2(bc(wu), B2b[1], fma2(bc(wd), B0b[1], B1b[1]));
-    const P2 Gb = fma2(bc(wu), B2b[2], fma2(bc(wd), B0b[2], B1b[2]));
-    float d0v[2], d1v[2], d2v[2];
-#pragma unroll
-    for (int f = 0; f < 2; ++f) {
-      const F4 sp = st.at(slot, 1 + 3 * f, C::STASH4);
-      const F4 sdx = st.at(slot, 2 + 3 * f, C::STASH4);
-      const F4 sdy = st.at(slot, 3 + 3 * f, C::STASH4);
-      const bool won = (L.tag1 == f);
-      const P2 A = fma2(bc(wu), B2rg[f][0], fma2(bc(wd), B0rg[f][0], B1rg[f][0]));
-      const P2 Bq = fma2(bc(wu), B2rg[f][1], fma2(bc(wd), B0rg[f][1], B1rg[f][1]));
-      const P2 G = fma2(bc(wu), B2rg[f][2], fma2(bc(wd), B0rg[f][2], B1rg[f][2]));
-      const P2 xrg = p2(sp.x, sp.y);
-      P2 grg = C::NOSSIM ? bc(0.f) : mul2(bc(0.85f / 3.0f), fma2(xrg, Bq, fma2(tgrg, G, A)));
-      float gb = C::NOSSIM ? 0.0f
-                           : (0.85f / 3.0f) * fmaf(sp.z, f ? Bb.y : Bb.x, fmaf(tgb, f ? Gb.y : Gb.x, f ? Ab.y : Ab.x));
-      if (won) {
-        const float mk = (!C::AUTOMASK && J.pm) ? MD2_LD(J.pm + f * J.plane + yp * J.W + L.xi) : 1.0f;
-        const float kl1 = (C::NOSSIM ? (1.0f / 3.0f) : (0.15f / 3.0f)) * mk;
-        const float dr = sp.x - tgrg.x, dg = sp.y - tgrg.y, db = sp.z - tgb;
-        grg.x += (dr != 0.f) ? copysignf(kl1, dr) : 0.0f;
-        grg.y += (dg != 0.f) ? copysignf(kl1, dg) : 0.0f;
-        gb += (db != 0.f) ? copysignf(kl1, db) : 0.0f;
-      }
-      float d0 = fmaf(grg.x, sdx.x, 0.f), d1 = fmaf(grg.x, sdy.x, 0.f);
-      d0 = fmaf(grg.y, sdx.y, d0); d1 = fmaf(grg.y, sdy.y, d1);
-      d0 = fmaf(gb, sdx.z, d0); d1 = fmaf(gb, sdy.z, d1);
-      d0v[f] = d0; d1v[f] = d1;
-      d2v[f] = -fmaf(sp.w, d0, sdx.w * d1);
-    }
-    const P2 d0 = p2(d0v[0], d0v[1]), d1 = p2(d1v[0], d1v[1]), d2 = p2(d2v[0], d2v[1]);
-    const P2 q0 = fma2(L.qb[0], bc(yf), L.qa[0]);
-    const P2 q1 = fma2(L.qb[1], bc(yf), L.qa[1]);
-    const P2 q2 = fma2(L.qb[2], bc(yf), L.qa[2]);
-    const P2 tt = fma2(d0, q0, fma2(d1, q1, mul2(d2, q2)));
-    const float dzsum = (0.f + tt.x) + tt.y;
-    const float zy = z * yf;
-    L.S1[0] = fma2(d0, bc(z), L.S1[0]); L.S1[1] = fma2(d1, bc(z), L.S1[1]); L.S1[2] = fma2(d2, bc(z), L.S1[2]);
-    L.S2[0] = fma2(d0, bc(zy), L.S2[0]); L.S2[1] = fma2(d1, bc(zy), L.S2[1]); L.S2[2] = fma2(d2, bc(zy), L.S2[2]);
-    L.S3[0] = add2(L.S3[0], d0); L.S3[1] = add2(L.S3[1], d1); L.S3[2] = add2(L.S3[2], d2);
-    const float dD = -P.c_disp * z * z * dzsum * P.gscale;
-    J.dD[yp * J.W + L.xi] = dD;
-    if (J.s == 0)
-      J.gd0[yp * J.W + L.xi] = dD + J.sm_w * (MD2_LD(J.gn0 + yp * J.W + L.xi) * J.sm_inv_m - J.sm_dterm);
-  }
-#pragma unroll
-  for (int i = 0; i < 3; ++i) {
-#pragma unroll
-    for (int f = 0; f < 2; ++f) { L.B2rg[f][i] = L.B1rg[f][i]; L.B1rg[f][i] = B0rg[f][i]; }
-    L.B2b[i] = L.B1b[i]; L.B1b[i] = B0b[i];
-  }
-  L.tag1 = L.tag;
 }
 
 // lane's share of dP for source f (see lane_dP)
