@@ -301,6 +301,46 @@ typedef struct md2_color_jitter {
 int md2_color_jitter_u8(const unsigned char *in, unsigned char *out, const md2_color_jitter *params, void *scratch,
                         size_t scratch_bytes, int n_images, int height, int width, int hwc, void *stream);
 
+/* ---- the training batch of MonoDataset.__getitem__ + preprocess on the GPU (SURVEY.md 8f-3,
+ * datasets/mono_dataset.py:90-109,136-185, kitti_dataset.py get_color): from the native uint8 frames a worker loaded,
+ * the flip, the LANCZOS pyramid and the per-scale colour augmentation of every (sample, frame) image of a batch, in
+ * 2 * num_scales + 3 launches whatever the batch size, frame count and mix of native sizes.
+ *
+ * Image n of a batch is described by a job.  Its native frame is (height, width, 3) uint8 HWC (np.array of the PIL
+ * image) at byte `offset` of `frames`; `flip` mirrors it horizontally before the resize (get_color's
+ * transpose(FLIP_LEFT_RIGHT)); `sample` is its row of `params` (one md2_color_jitter per dataset item, shared by its
+ * frames and scales; a row whose order is all -1 is the identity); `size` is the index
+ * md2_batch_plan_add_native_size returned for (height, width).
+ *
+ * Outputs hold every level back to back: level s (h_s = height >> s, w_s = width >> s) starts at element
+ * n_images * 3 * sum_{t<s} h_t * w_t, image n of it at n * 3 * h_s * w_s, NCHW.
+ *   out_color:     ("color", f, s): the resized bytes, uint8, or float32 x / 255 (= ToTensor) when color_f32 != 0;
+ *   out_color_aug: ("color_aug", f, s): float32 ToTensor of the jittered level (the jitter runs after each resize, with
+ *                  the level's own contrast mean, as the reference's preprocess does).
+ * Creating the plan and adding a size are synchronous (tables are built on the host in double arithmetic, as Pillow
+ * does, and uploaded); md2_batch_build_u8 only enqueues, so once every native size is added it can be captured in a
+ * CUDA graph.  `jobs` is read on the host for validation, `jobs_dev` (the same records on the device) by the kernels. */
+#define MD2_BATCH_MAX_SIZES 64
+typedef struct md2_batch_job {
+  long long offset;           /* byte offset of the native frame in `frames` */
+  int height, width;          /* native size */
+  int size;                   /* index of (height, width) in the plan */
+  int flip;                   /* non-zero: mirrored (do_flip) */
+  int sample;                 /* row of `params` */
+  int reserved;
+} md2_batch_job;
+typedef struct md2_batch_plan md2_batch_plan;
+int md2_batch_plan_create(int height, int width, int num_scales, md2_batch_plan **plan);
+void md2_batch_plan_destroy(md2_batch_plan *plan);
+/* index of (h, w) among the plan's native sizes; tables are built and uploaded the first time a size is added */
+int md2_batch_plan_add_native_size(md2_batch_plan *plan, int h, int w, int *index);
+/* bytes of device scratch one md2_batch_build_u8 call over n_images needs */
+int md2_batch_scratch_bytes(const md2_batch_plan *plan, int n_images, int color_f32, size_t *bytes);
+int md2_batch_build_u8(const md2_batch_plan *plan, const unsigned char *frames, size_t frames_bytes,
+                       const md2_batch_job *jobs, const md2_batch_job *jobs_dev, int n_images,
+                       const md2_color_jitter *params, int n_samples, void *out_color, int color_f32,
+                       float *out_color_aug, void *scratch, size_t scratch_bytes, void *stream);
+
 #ifdef __cplusplus
 }
 #endif

@@ -84,6 +84,8 @@ SYMBOLS = [
     "md2_dispconv_sigmoid_typed", "md2_dispconv_sigmoid_backward_typed",
     "md2_resize_plan_create", "md2_resize_plan_destroy", "md2_resize_scratch_bytes", "md2_resize_lanczos_u8",
     "md2_color_jitter_u8", "md2_upcat_pad", "md2_upcat_pad_backward",
+    "md2_batch_plan_create", "md2_batch_plan_destroy", "md2_batch_plan_add_native_size", "md2_batch_scratch_bytes",
+    "md2_batch_build_u8",
 ]
 
 _lib = None
@@ -111,7 +113,7 @@ def load_library(path: str = None) -> C.CDLL:
     lib.md2_view_synthesis_loss.argtypes = [C.POINTER(Md2Problem), C.POINTER(Md2Tensors), C.c_void_p,
                                             C.c_size_t, C.c_void_p]
     for name in SYMBOLS:
-        if name not in ("md2_status_string", "md2_resize_plan_destroy") and hasattr(lib, name):
+        if name not in ("md2_status_string", "md2_resize_plan_destroy", "md2_batch_plan_destroy") and hasattr(lib, name):
             getattr(lib, name).restype = C.c_int
     lib.md2_scale_tensors.argtypes = [C.c_int, C.POINTER(C.c_void_p), C.POINTER(C.c_void_p), C.POINTER(C.c_longlong),
                                       C.c_void_p, C.c_void_p]
@@ -131,6 +133,13 @@ def load_library(path: str = None) -> C.CDLL:
                                         C.c_int, C.c_int, C.c_void_p]
     lib.md2_resize_lanczos_u8.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_size_t, C.c_int,
                                           C.c_int, C.c_void_p]
+    lib.md2_batch_plan_create.argtypes = [C.c_int, C.c_int, C.c_int, C.POINTER(C.c_void_p)]
+    lib.md2_batch_plan_destroy.restype = None
+    lib.md2_batch_plan_destroy.argtypes = [C.c_void_p]
+    lib.md2_batch_plan_add_native_size.argtypes = [C.c_void_p, C.c_int, C.c_int, C.POINTER(C.c_int)]
+    lib.md2_batch_scratch_bytes.argtypes = [C.c_void_p, C.c_int, C.c_int, C.POINTER(C.c_size_t)]
+    lib.md2_batch_build_u8.argtypes = [C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p, C.c_void_p, C.c_int, C.c_void_p,
+                                       C.c_int, C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p]
     if path is None:
         _lib = lib
     return lib
