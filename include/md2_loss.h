@@ -341,6 +341,42 @@ int md2_batch_build_u8(const md2_batch_plan *plan, const unsigned char *frames, 
                        const md2_color_jitter *params, int n_samples, void *out_color, int color_f32,
                        float *out_color_aug, void *scratch, size_t scratch_bytes, void *stream);
 
+/* ---- KITTI raw depth_gt on the GPU (SURVEY.md 8f-3): KITTIRAWDataset.get_depth (datasets/kitti_dataset.py) =
+ * generate_depth_map (kitti_utils.py) + skimage.transform.resize(order=0, preserve_range=True, mode='constant')
+ * to (out_h, out_w) + np.fliplr when flipped, then the float32 rounding of MonoDataset.__getitem__.
+ *
+ * Job n is one sample.  Its scan is the velodyne file as read: n_points x 4 float32 (x, y, z, reflectance; the 4th
+ * column is ignored) at byte `offset` of `scans`, 16-byte aligned.  P is P_velo2im (row-major 3x4, float64) and
+ * (height, width) the native image size im_shape, both from the drive's calibration (host code, cached per camera).
+ * Per point, in float64: (u', v', w) = P (x, y, z, 1), col = rint(u'/w) - 1, row = rint(v'/w) - 1; points with x >= 0
+ * landing inside the native image store w (x when vel_depth != 0); the last point at a pixel wins, then each group of
+ * the reference's sub2ind (a pixel, plus (r+1, 0) for (r, W-1)) holding more than one point gets the group's minimum
+ * at the pixel of its first point; negatives become 0.  The order-0 resize takes output o from native index
+ * floor((o + 0.5) * (n / n_out) - 0.5 + 0.5) (float64, in that order).  out: (n_jobs, 1, out_h, out_w) float32.
+ * An output size equal to the native size gives generate_depth_map itself (export_gt_depth.py's use).
+ *
+ * Every native axis must be shorter than 1.25 x the output axis (beyond that skimage's anti-aliasing filter smooths
+ * the map) and the native width at least 2: else MD2_ERR_UNSUPPORTED.  `jobs` is read on the host for validation,
+ * `jobs_dev` (the same records on the device) by the kernels.  The scratch size depends only on n_jobs and the output
+ * size, and md2_velo_depth only enqueues (3 launches), so one allocation and one captured CUDA graph serve every batch
+ * of that shape.  Bitwise reproducible.
+ * The maps are the reference's bit for bit with one exception: a zero is always +0.0.  The reference keeps a -0.0 stored
+ * value (only a velodyne x of -0.0 under vel_depth gives one) through some of numpy's reductions and clips and not
+ * others, so its sign there depends on numpy's summation order. ---- */
+typedef struct md2_velo_job {
+  double P[12];               /* P_velo2im, row-major 3x4 */
+  long long offset;           /* byte offset of the scan in `scans` */
+  int n_points;               /* rows of the scan */
+  int height, width;          /* native image size (im_shape) */
+  int flip;                   /* non-zero: np.fliplr after the resize (do_flip) */
+  int vel_depth;              /* non-zero: store the velodyne x instead of the camera depth */
+  int reserved;
+} md2_velo_job;
+int md2_velo_depth_scratch_bytes(int n_jobs, int out_h, int out_w, size_t *bytes);
+int md2_velo_depth(const unsigned char *scans, size_t scans_bytes, const md2_velo_job *jobs,
+                   const md2_velo_job *jobs_dev, int n_jobs, float *out, int out_h, int out_w, void *scratch,
+                   size_t scratch_bytes, void *stream);
+
 #ifdef __cplusplus
 }
 #endif

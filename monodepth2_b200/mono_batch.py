@@ -23,7 +23,7 @@ from typing import Dict, List, Optional
 import numpy as np
 import torch
 
-from . import _capi
+from . import _capi, kitti_depth
 from .pyramid import ColorAug
 
 # KITTIDataset.K (kitti_dataset.py): intrinsics normalised by the image size
@@ -37,7 +37,7 @@ JOB_DTYPE = np.dtype([("offset", "<i8"), ("height", "<i4"), ("width", "<i4"), ("
                       ("sample", "<i4"), ("reserved", "<i4")])
 _PARAM_BYTES = 32           # one md2_color_jitter row
 _STEREO_BYTES = 64          # one 4x4 float32 stereo_T
-_DRAW_KEYS = ("frames", "do_color_aug", "do_flip", "color_aug", "side")
+_DRAW_KEYS = ("frames", "do_color_aug", "do_flip", "color_aug", "side", "velodyne")
 
 
 def _align(n: int, a: int = 16) -> int:
@@ -50,7 +50,10 @@ class NativeBatch:
     layout, one per sample), the stereo_T matrices (when ``"s"`` is a frame), the job table (``JOB_DTYPE``, image
     ``fi * batch_size + b`` is frame ``frame_ids[fi]`` of sample ``b``) and the native HWC frames.  The draws stay
     readable: ``do_color_aug`` / ``do_flip`` (B,) bool, ``color_aug`` the ``ColorJitter.get_params`` tuple or None per
-    sample, ``side`` per sample; ``extra`` holds the dataset's other keys (``depth_gt``), default-collated."""
+    sample, ``side`` per sample; ``extra`` holds the dataset's other keys (``depth_gt``), default-collated.  Items from
+    ``VelodyneDepthMixin`` add the ``md2_velo_job`` table at ``velo_jobs_offset``, between the frames' job table and the
+    frames (so, like every other offset but the scans', it depends only on the batch size and the frame ids), and the
+    scans after the frames; ``velo_out_shape`` is the size of the depth_gt they give."""
     buffer: torch.Tensor
     batch_size: int
     frame_ids: list
@@ -63,6 +66,8 @@ class NativeBatch:
     color_aug: list
     side: list
     extra: dict
+    velo_jobs_offset: int = -1  # -1 without velodyne scans
+    velo_out_shape: Optional[tuple] = None
 
     @property
     def n_images(self) -> int:
@@ -98,11 +103,22 @@ def collate_native(items: List[dict], pin_memory: Optional[bool] = None) -> Nati
     stereo_off = off if stereo else -1
     off += B * _STEREO_BYTES if stereo else 0
     jobs_off = off
-    frames_off = _align(off + n * JOB_DTYPE.itemsize)
+    off = _align(off + n * JOB_DTYPE.itemsize)
+    velo = [it["velodyne"] for it in items] if "velodyne" in items[0] else None
+    velo_off = -1
+    if velo is not None:        # the scans' job table ahead of the frames: its offset depends on B alone, so a graph
+        if any(tuple(v.out_shape) != tuple(velo[0].out_shape) for v in velo):    # captured on one batch serves all
+            raise ValueError("every velodyne scan of a batch must give the same depth_gt size")
+        velo_off = off
+        off = _align(off + B * kitti_depth.VELO_JOB_DTYPE.itemsize)
+    frames_off = off
     rel, total = [], 0
     for a in frames:
         rel.append(total)
         total = _align(total + a.nbytes)
+    if velo is not None:        # the scans after the frames; their job records hold their offsets
+        scans_off = frames_off + total
+        total += kitti_depth.packed_bytes(velo)
     if pin_memory is None:
         pin_memory = get_worker_info() is None and torch.cuda.is_available()
     buf = torch.empty(frames_off + total, dtype=torch.uint8, pin_memory=bool(pin_memory))
@@ -125,10 +141,13 @@ def collate_native(items: List[dict], pin_memory: Optional[bool] = None) -> Nati
     for i, a in enumerate(frames):
         jobs[i] = (rel[i], a.shape[0], a.shape[1], -1, int(do_flip[i % B]), i % B, 0)
         h[frames_off + rel[i]:frames_off + rel[i] + a.nbytes] = a.reshape(-1)
+    if velo is not None:
+        kitti_depth.pack_jobs(h, velo_off, scans_off, velo, do_flip, False)
     extra_keys = [k for k in items[0] if k not in _DRAW_KEYS]
     extra = default_collate([{k: it[k] for k in extra_keys} for it in items]) if extra_keys else {}
     return NativeBatch(buf, B, fids, 0, stereo_off, jobs_off, frames_off,
-                       torch.tensor([bool(it["do_color_aug"]) for it in items]), torch.tensor(do_flip), draws, sides, extra)
+                       torch.tensor([bool(it["do_color_aug"]) for it in items]), torch.tensor(do_flip), draws, sides, extra,
+                       velo_off, tuple(velo[0].out_shape) if velo is not None else None)
 
 
 class NativeFramesMixin:
@@ -137,7 +156,8 @@ class NativeFramesMixin:
     ``__getitem__`` makes the reference's random draws in the reference's order (mono_dataset.py:136-185: do_color_aug,
     do_flip, then ``ColorJitter.get_params`` only when augmenting) and loads every frame with the dataset's own
     ``get_color(folder, index, side, False)``, unflipped and unresized: the flip, the pyramid and the jitter run in
-    ``MonoBatch``.  ``depth_gt`` stays the reference's host code."""
+    ``MonoBatch``.  ``depth_gt`` is the dataset's own host code (``native_depth``), unless ``VelodyneDepthMixin`` is
+    put in front."""
 
     def __getitem__(self, index):
         from torchvision import transforms
@@ -159,17 +179,22 @@ class NativeFramesMixin:
             color_aug = transforms.ColorJitter.get_params(self.brightness, self.contrast, self.saturation, self.hue)
         item = {"frames": frames, "do_color_aug": bool(do_color_aug), "do_flip": bool(do_flip), "color_aug": color_aug,
                 "side": side}
-        if self.load_depth:    # as MonoDataset.__getitem__ does
-            depth_gt = self.get_depth(folder, frame_index, side, do_flip)
-            item["depth_gt"] = torch.from_numpy(np.expand_dims(depth_gt, 0).astype(np.float32))
+        if self.load_depth:
+            item.update(self.native_depth(folder, frame_index, side, do_flip))
         return item
+
+    def native_depth(self, folder, frame_index, side, do_flip) -> dict:
+        """The item's depth keys: ``depth_gt`` from the dataset's ``get_depth``, as MonoDataset.__getitem__ does."""
+        depth_gt = self.get_depth(folder, frame_index, side, do_flip)
+        return {"depth_gt": torch.from_numpy(np.expand_dims(depth_gt, 0).astype(np.float32))}
 
 
 class MonoBatch:
     """``MonoBatch(height, width, frame_ids, num_scales)(native) -> inputs`` with the keys and shapes default collation of
     ``MonoDataset.__getitem__`` gives: ``("color", f, s)`` (B,3,h_s,w_s) uint8 (or float32 ``ToTensor`` values with
     ``color_dtype=torch.float32``), ``("color_aug", f, s)`` float32, ``("K", s)`` / ``("inv_K", s)`` (B,4,4) float32,
-    ``"stereo_T"`` when ``"s"`` is a frame, and the dataset's other keys.  uint8 ``color`` is what the fused loss's uint8
+    ``"stereo_T"`` when ``"s"`` is a frame, ``"depth_gt"`` built from the scans (``md2_velo_depth``, three launches) when
+    the items came from ``VelodyneDepthMixin``, and the dataset's other keys.  uint8 ``color`` is what the fused loss's uint8
     entry takes.  The K / inv_K tensors are shared between calls with the same batch size: treat them as read-only.
 
     The first batch that holds a new native size builds that size's tables (synchronous); after that a call only
@@ -266,6 +291,9 @@ class MonoBatch:
             off += 3 * n * planes[s]
         for k, v in native.extra.items():
             inputs[k] = v.to(dev, non_blocking=True) if torch.is_tensor(v) else v
+        if native.velo_jobs_offset >= 0:
+            inputs["depth_gt"] = kitti_depth.run(self.lib, flat, native.buffer.data_ptr() + native.velo_jobs_offset,
+                                                 native.velo_jobs_offset, B, native.velo_out_shape)
         if native.stereo_offset >= 0:
             a = native.stereo_offset
             inputs["stereo_T"] = flat[a:a + B * _STEREO_BYTES].view(torch.float32).view(B, 4, 4)

@@ -150,3 +150,60 @@ def make_batch(batch: int = 12, height: int = 192, width: int = 640,
                                              W >> (s if multiscale_noise else 0), generator=gn)
                                  for s in range(num_scales)]
     return inputs, outputs, pose, noise
+
+
+# ---- KITTI raw velodyne scans and calibration (depth_gt on the GPU, monodepth2_b200/kitti_depth.py)
+# The 2011_09_26 calibration published with KITTI raw, rounded as its text files print it.
+KITTI_CAM_TO_CAM = {
+    "R_rect_00": [9.999239e-01, 9.837760e-03, -7.445048e-03, -9.869795e-03, 9.999421e-01, -4.278459e-03,
+                  7.402527e-03, 4.351614e-03, 9.999631e-01],
+    "P_rect_02": [7.215377e+02, 0.0, 6.095593e+02, 4.485728e+01, 0.0, 7.215377e+02, 1.728540e+02, 2.163791e-01,
+                  0.0, 0.0, 1.0, 2.745884e-03],
+    "P_rect_03": [7.215377e+02, 0.0, 6.095593e+02, -3.395242e+02, 0.0, 7.215377e+02, 1.728540e+02, 2.199936e+00,
+                  0.0, 0.0, 1.0, 2.729905e-03],
+}
+KITTI_VELO_TO_CAM = {
+    "R": [7.533745e-03, -9.999714e-01, -6.166020e-04, 1.480249e-02, 7.280733e-04, -9.998902e-01, 9.998621e-01,
+          7.523790e-03, 1.480755e-02],
+    "T": [-4.069766e-03, -7.631618e-02, -2.717806e-01],
+}
+KITTI_NATIVE_SIZES = [(375, 1242), (376, 1241), (374, 1238), (370, 1226), (370, 1224)]    # (h, w) of the raw drives
+
+
+def write_kitti_calibration(calib_dir: str, im_shape=(375, 1242), cam_to_cam: dict = None, velo_to_cam: dict = None):
+    """calib_cam_to_cam.txt and calib_velo_to_cam.txt in KITTI's text format (``key: v v v`` in %.6e where that is exact,
+    and a calib_time line that read_calib_file keeps as a string)."""
+    import os
+    cc = dict(KITTI_CAM_TO_CAM if cam_to_cam is None else cam_to_cam)
+    vc = dict(KITTI_VELO_TO_CAM if velo_to_cam is None else velo_to_cam)
+    fmt = lambda vals: " ".join("%.6e" % v if float("%.6e" % v) == v else repr(float(v)) for v in vals)
+    os.makedirs(calib_dir, exist_ok=True)
+    with open(os.path.join(calib_dir, "calib_cam_to_cam.txt"), "w") as f:
+        f.write("calib_time: 09-Jan-2012 13:57:47\ncorner_dist: 9.950000e-02\n")
+        f.write("S_rect_02: %s\nS_rect_03: %s\n" % (fmt([im_shape[1], im_shape[0]]), fmt([im_shape[1], im_shape[0]])))
+        for k, v in cc.items():
+            f.write("%s: %s\n" % (k, fmt(v)))
+    with open(os.path.join(calib_dir, "calib_velo_to_cam.txt"), "w") as f:
+        f.write("calib_time: 15-Mar-2012 11:37:16\n")
+        for k, v in vc.items():
+            f.write("%s: %s\n" % (k, fmt(v)))
+        f.write("delta_f: 0.000000e+00 0.000000e+00\ndelta_c: 0.000000e+00 0.000000e+00\n")
+
+
+def velodyne_scan(seed: int, n_azimuth: int = 1900, n_beams: int = 64) -> np.ndarray:
+    """A KITTI-like HDL-64 sweep, (n_beams * n_azimuth, 4) float32 (x forward, y left, z up, reflectance): a ground
+    plane 1.73 m below the sensor and walls of a street, ranges clipped to 120 m, range noise, and a few dropped
+    returns (NaN).  About a seventh of the points fall inside the left camera's image."""
+    rng = np.random.default_rng(seed)
+    az = np.linspace(-np.pi, np.pi, n_azimuth, endpoint=False) + rng.uniform(0, 2 * np.pi / n_azimuth)
+    el = np.deg2rad(np.linspace(2.0, -24.8, n_beams))
+    A, E = np.meshgrid(az, el)
+    d = np.stack([np.cos(E) * np.cos(A), np.cos(E) * np.sin(A), np.sin(E)], -1)
+    ground = np.where(d[..., 2] < -1e-3, -1.73 / np.minimum(d[..., 2], -1e-3), np.inf)
+    wall = np.where(np.abs(d[..., 1]) > 1e-3, (7.0 + 2.0 * np.sin(3 * A)) / np.maximum(np.abs(d[..., 1]), 1e-3), np.inf)
+    r = np.minimum(np.minimum(ground, wall), 120.0) * (1 + rng.normal(0, 0.003, A.shape))
+    pts = (d * r[..., None]).reshape(-1, 3)
+    refl = rng.uniform(0, 1, (pts.shape[0], 1))
+    scan = np.concatenate([pts, refl], 1).astype(np.float32)
+    scan[rng.random(scan.shape[0]) < 0.002, :3] = np.nan
+    return scan
