@@ -377,6 +377,62 @@ int md2_velo_depth(const unsigned char *scans, size_t scans_bytes, const md2_vel
                    const md2_velo_job *jobs_dev, int n_jobs, float *out, int out_h, int out_w, void *scratch,
                    size_t scratch_bytes, void *stream);
 
+/* ---- baseline JPEG decoding on the GPU: the frames of kitti_dataset.py get_color, pil_loader's
+ * Image.open(f).convert("RGB"), byte for byte what Pillow's libjpeg-turbo gives, for SOF0 8-bit Huffman-coded
+ * three-component YCbCr streams with luma sampling 1x1, 2x1 or 2x2 and chroma 1x1, any restart interval.
+ *
+ * The host (monodepth2_b200/jpeg.py) walks the markers, removes the 0xFF00 stuffing and the RSTn markers, and lays
+ * out per image, inside `data`: the entropy-coded segments (one per restart interval), each starting on a
+ * MD2_JPEG_CHUNK_BYTES boundary of the image's entropy area and zero-padded to the next; the segment table
+ * (n_segments md2_jpeg_segment); and an md2_jpeg_tables record (several images may share one).
+ * Chunks are numbered across the call: image n owns chunks [chunk_offset, chunk_offset + n_chunks), and blocks
+ * [block_offset, block_offset + mcus * blocks per MCU) of the coefficient scratch; both offsets are the running sums
+ * over the images before it.  The image is written as (height, width, 3) uint8 HWC at byte out_offset of `frames`.
+ *
+ * status (device, n_images uint32) gets per image the MD2_JPEG_* bits below; 0 is a clean decode.  A stream that sets
+ * one may leave any bytes in its frame, but the call never reads or writes outside its buffers.
+ * The scratch size depends only on n_images and the capacity (max_chunks, max_blocks); md2_jpeg_decode only enqueues
+ * (a memset and four kernels), so one allocation and one captured CUDA graph serve every batch within the capacity.
+ * `jobs` is read on the host for validation, `jobs_dev` (the same records on the device) by the kernels. ---- */
+#define MD2_JPEG_CHUNK_BYTES 64
+#define MD2_JPEG_BAD_CODE 1u          /* a Huffman code no table holds */
+#define MD2_JPEG_EXHAUSTED 2u         /* a segment's data ended before its last MCU */
+#define MD2_JPEG_BAD_INDEX 4u         /* a run took the coefficient index past 63 */
+#define MD2_JPEG_BAD_SEGMENT 8u       /* a segment record outside the image's chunks */
+typedef struct md2_jpeg_huff {        /* jpeg_make_d_derived_tbl */
+  unsigned short look[256];           /* (code length << 8) | symbol for codes of <= 8 bits, else 0 */
+  int maxcode[18];                    /* largest code of each length, -1 if none; maxcode[17] = 0xFFFFF */
+  int valoffset[18];                  /* huffval index = code + valoffset[length] */
+  unsigned char huffval[256];
+} md2_jpeg_huff;
+typedef struct md2_jpeg_tables {
+  md2_jpeg_huff dc[2], ac[2];
+  unsigned short quant[4][64];        /* natural (row-major) order */
+} md2_jpeg_tables;
+typedef struct md2_jpeg_segment {
+  int chunk;                          /* first chunk, counted from the image's first */
+  int bytes;                          /* unstuffed entropy bytes */
+} md2_jpeg_segment;
+typedef struct md2_jpeg_job {
+  long long out_offset;               /* byte offset of the decoded frame in `frames` */
+  long long entropy_offset;           /* byte offset of the image's entropy area (its chunk 0) in `data` */
+  long long segments_offset;          /* byte offset of the segment table in `data`, 8-byte aligned */
+  long long tables_offset;            /* byte offset of the md2_jpeg_tables record in `data`, 8-byte aligned */
+  long long block_offset;             /* first block in the coefficient scratch */
+  int chunk_offset, n_chunks;         /* the image's chunks */
+  int n_segments;                     /* ceil(mcus / restart_interval), 1 without restart interval */
+  int restart_interval;               /* MCUs per segment, 0: one segment */
+  int height, width;
+  int h_samp, v_samp;                 /* luma sampling: (1, 1), (2, 1) or (2, 2) */
+  int dc_table[3], ac_table[3];       /* 0 or 1 per component (Y, Cb, Cr) */
+  int quant_table[3];                 /* 0..3 per component */
+  int reserved;
+} md2_jpeg_job;
+int md2_jpeg_decode_scratch_bytes(int n_images, long long max_chunks, long long max_blocks, size_t *bytes);
+int md2_jpeg_decode(const unsigned char *data, size_t data_bytes, const md2_jpeg_job *jobs, const md2_jpeg_job *jobs_dev,
+                    int n_images, unsigned char *frames, size_t frames_bytes, unsigned int *status,
+                    long long max_chunks, long long max_blocks, void *scratch, size_t scratch_bytes, void *stream);
+
 #ifdef __cplusplus
 }
 #endif

@@ -86,6 +86,7 @@ SYMBOLS = [
     "md2_color_jitter_u8", "md2_upcat_pad", "md2_upcat_pad_backward",
     "md2_batch_plan_create", "md2_batch_plan_destroy", "md2_batch_plan_add_native_size", "md2_batch_scratch_bytes",
     "md2_batch_build_u8", "md2_velo_depth_scratch_bytes", "md2_velo_depth",
+    "md2_jpeg_decode_scratch_bytes", "md2_jpeg_decode",
 ]
 
 _lib = None
@@ -143,6 +144,9 @@ def load_library(path: str = None) -> C.CDLL:
     lib.md2_velo_depth_scratch_bytes.argtypes = [C.c_int, C.c_int, C.c_int, C.POINTER(C.c_size_t)]
     lib.md2_velo_depth.argtypes = [C.c_void_p, C.c_size_t, C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.c_int, C.c_int,
                                    C.c_void_p, C.c_size_t, C.c_void_p]
+    lib.md2_jpeg_decode_scratch_bytes.argtypes = [C.c_int, C.c_longlong, C.c_longlong, C.POINTER(C.c_size_t)]
+    lib.md2_jpeg_decode.argtypes = [C.c_void_p, C.c_size_t, C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.c_size_t,
+                                    C.c_void_p, C.c_longlong, C.c_longlong, C.c_void_p, C.c_size_t, C.c_void_p]
     if path is None:
         _lib = lib
     return lib

@@ -23,7 +23,7 @@ from typing import Dict, List, Optional
 import numpy as np
 import torch
 
-from . import _capi, kitti_depth
+from . import _capi, jpeg, kitti_depth
 from .pyramid import ColorAug
 
 # KITTIDataset.K (kitti_dataset.py): intrinsics normalised by the image size
@@ -68,6 +68,17 @@ class NativeBatch:
     extra: dict
     velo_jobs_offset: int = -1  # -1 without velodyne scans
     velo_out_shape: Optional[tuple] = None
+    # Items from JpegFramesMixin: the md2_jpeg_job table of the JPEG frames at jpeg_jobs_offset (after the scans' job
+    # table, so its place depends only on the batch size and the frame ids), their compressed streams after the
+    # frames and scans.  The job table's frame offsets then index a device native-frame buffer of native_bytes, into
+    # which the JPEG frames are decoded and the host-decoded frames (jpeg_copies: (offset in buffer, offset in that
+    # device buffer, bytes)) are copied.
+    jpeg_jobs_offset: int = -1
+    jpeg_names: Optional[list] = None
+    jpeg_chunks: int = 0
+    jpeg_blocks: int = 0
+    native_bytes: int = 0
+    jpeg_copies: Optional[list] = None
 
     @property
     def n_images(self) -> int:
@@ -94,8 +105,12 @@ def collate_native(items: List[dict], pin_memory: Optional[bool] = None) -> Nati
         if list(it["frames"].keys()) != fids:
             raise ValueError("every item of a batch must hold the same frame ids")
     n = B * len(fids)
-    frames = [np.ascontiguousarray(items[b]["frames"][f], dtype=np.uint8) for f in fids for b in range(B)]
+    frames = [items[b]["frames"][f] for f in fids for b in range(B)]
+    frames = [a if isinstance(a, jpeg.JpegStream) else np.ascontiguousarray(a, dtype=np.uint8) for a in frames]
+    streams = [a for a in frames if isinstance(a, jpeg.JpegStream)]
     for a in frames:
+        if isinstance(a, jpeg.JpegStream):
+            continue
         if a.ndim != 3 or a.shape[2] != 3:
             raise ValueError("native frames must be (h, w, 3) uint8 arrays, got %s" % (a.shape,))
     stereo = "s" in fids
@@ -111,14 +126,29 @@ def collate_native(items: List[dict], pin_memory: Optional[bool] = None) -> Nati
             raise ValueError("every velodyne scan of a batch must give the same depth_gt size")
         velo_off = off
         off = _align(off + B * kitti_depth.VELO_JOB_DTYPE.itemsize)
+    jpeg_off = -1
+    if streams:
+        jpeg_off = off
+        off = _align(off + len(streams) * jpeg.JOB_DTYPE.itemsize, 64)
     frames_off = off
     rel, total = [], 0
     for a in frames:
         rel.append(total)
         total = _align(total + a.nbytes)
+    native_total = total
+    copies = None
+    if streams:                 # the buffer holds only the host-decoded frames; rel indexes the device frame buffer
+        copies, total = [], 0
+        for a, r in zip(frames, rel):
+            if not isinstance(a, jpeg.JpegStream):
+                copies.append((frames_off + total, r, a.nbytes))
+                total = _align(total + a.nbytes)
     if velo is not None:        # the scans after the frames; their job records hold their offsets
         scans_off = frames_off + total
         total += kitti_depth.packed_bytes(velo)
+    if streams:
+        body_off = _align(frames_off + total, 64)
+        total = body_off - frames_off + jpeg.body_bytes(streams)
     if pin_memory is None:
         pin_memory = get_worker_info() is None and torch.cuda.is_available()
     buf = torch.empty(frames_off + total, dtype=torch.uint8, pin_memory=bool(pin_memory))
@@ -140,14 +170,24 @@ def collate_native(items: List[dict], pin_memory: Optional[bool] = None) -> Nati
     jobs = h[jobs_off:jobs_off + n * JOB_DTYPE.itemsize].view(JOB_DTYPE)
     for i, a in enumerate(frames):
         jobs[i] = (rel[i], a.shape[0], a.shape[1], -1, int(do_flip[i % B]), i % B, 0)
-        h[frames_off + rel[i]:frames_off + rel[i] + a.nbytes] = a.reshape(-1)
+    if copies is None:
+        for a, r in zip(frames, rel):
+            h[frames_off + r:frames_off + r + a.nbytes] = a.reshape(-1)
+    else:
+        for a, (src, _, nb) in zip([a for a in frames if not isinstance(a, jpeg.JpegStream)], copies):
+            h[src:src + nb] = a.reshape(-1)
     if velo is not None:
         kitti_depth.pack_jobs(h, velo_off, scans_off, velo, do_flip, False)
+    chunks = blocks = 0
+    if streams:
+        chunks, blocks = jpeg.pack(h, jpeg_off, body_off, streams,
+                                   [r for a, r in zip(frames, rel) if isinstance(a, jpeg.JpegStream)])
     extra_keys = [k for k in items[0] if k not in _DRAW_KEYS]
     extra = default_collate([{k: it[k] for k in extra_keys} for it in items]) if extra_keys else {}
     return NativeBatch(buf, B, fids, 0, stereo_off, jobs_off, frames_off,
                        torch.tensor([bool(it["do_color_aug"]) for it in items]), torch.tensor(do_flip), draws, sides, extra,
-                       velo_off, tuple(velo[0].out_shape) if velo is not None else None)
+                       velo_off, tuple(velo[0].out_shape) if velo is not None else None, jpeg_off,
+                       [s.name for s in streams], chunks, blocks, native_total, copies)
 
 
 class NativeFramesMixin:
@@ -171,9 +211,9 @@ class NativeFramesMixin:
         for i in self.frame_idxs:
             if i == "s":
                 other_side = {"r": "l", "l": "r"}[side]
-                frames[i] = np.array(self.get_color(folder, frame_index, other_side, False))
+                frames[i] = self.native_color(folder, frame_index, other_side)
             else:
-                frames[i] = np.array(self.get_color(folder, frame_index + i, side, False))
+                frames[i] = self.native_color(folder, frame_index + i, side)
         color_aug = None
         if do_color_aug:       # a tuple in the installed torchvision (SURVEY.md B.2); MonoBatch applies it
             color_aug = transforms.ColorJitter.get_params(self.brightness, self.contrast, self.saturation, self.hue)
@@ -182,6 +222,11 @@ class NativeFramesMixin:
         if self.load_depth:
             item.update(self.native_depth(folder, frame_index, side, do_flip))
         return item
+
+    def native_color(self, folder, frame_index, side):
+        """A native frame: the dataset's ``get_color(folder, frame_index, side, False)`` as an (h, w, 3) uint8 array
+        (``JpegFramesMixin`` returns the parsed JPEG instead)."""
+        return np.array(self.get_color(folder, frame_index, side, False))
 
     def native_depth(self, folder, frame_index, side, do_flip) -> dict:
         """The item's depth keys: ``depth_gt`` from the dataset's ``get_depth``, as MonoDataset.__getitem__ does."""
@@ -198,10 +243,18 @@ class MonoBatch:
     entry takes.  The K / inv_K tensors are shared between calls with the same batch size: treat them as read-only.
 
     The first batch that holds a new native size builds that size's tables (synchronous); after that a call only
-    enqueues work, and ``build`` alone can be captured in a CUDA graph."""
+    enqueues work, and ``build`` alone can be captured in a CUDA graph.
+
+    Batches of ``JpegFramesMixin`` items are decoded on the device first (``md2_jpeg_decode``) into a native-frame
+    buffer.  ``jpeg_capacity = (native_bytes, entropy_bytes, blocks)`` sizes that buffer and the decoder's scratch
+    (``entropy_bytes`` counts each restart segment rounded up to whole 64-byte chunks, as ``collate_native`` lays them
+    out); a batch over it raises before anything is enqueued.  With a capacity, a graph captured on one batch replays
+    batches of other compressed lengths and native sizes that hold as many JPEG frames and no host-decoded frame;
+    without, each batch is sized to itself.  ``jpeg_status`` is the device status word of every JPEG frame of the last
+    build (read without synchronising); ``check_jpeg()`` synchronises and raises naming the corrupt files."""
 
     def __init__(self, height: int, width: int, frame_ids, num_scales: int = 4, K=None,
-                 color_dtype: torch.dtype = torch.uint8, device=None):
+                 color_dtype: torch.dtype = torch.uint8, device=None, jpeg_capacity=None):
         if color_dtype not in (torch.uint8, torch.float32):
             raise ValueError("color_dtype must be torch.uint8 or torch.float32")
         self.height, self.width, self.num_scales = int(height), int(width), int(num_scales)
@@ -222,6 +275,9 @@ class MonoBatch:
             Ks[1, :] *= self.height // (2 ** scale)
             self._K.append((Ks, np.linalg.pinv(Ks)))
         self._k_cache: Dict[int, dict] = {}
+        self.jpeg_capacity = None if jpeg_capacity is None else tuple(int(v) for v in jpeg_capacity)
+        self.jpeg_status: Optional[torch.Tensor] = None
+        self._jpeg_names: list = []
 
     def __del__(self):
         try:
@@ -272,9 +328,13 @@ class MonoBatch:
         _capi.check(self.lib, self.lib.md2_batch_scratch_bytes(self._plan, n, f32, C.byref(nb)), "md2_batch_scratch_bytes")
         scratch = torch.empty(nb.value, dtype=torch.uint8, device=dev)
         base = flat.data_ptr()
+        frames_ptr, frames_bytes = base + native.frames_offset, flat.numel() - native.frames_offset
+        if native.jpeg_jobs_offset >= 0:
+            frames = self._decode_jpeg(native, flat)
+            frames_ptr, frames_bytes = frames.data_ptr(), frames.numel()
         with torch.cuda.device(dev):
             st = self.lib.md2_batch_build_u8(
-                self._plan, base + native.frames_offset, flat.numel() - native.frames_offset,
+                self._plan, frames_ptr, frames_bytes,
                 native.buffer.data_ptr() + native.jobs_offset, base + native.jobs_offset, n,
                 base + native.params_offset, B, color.data_ptr(), f32, color_aug.data_ptr(), scratch.data_ptr(),
                 scratch.numel(), C.c_void_p(torch.cuda.current_stream().cuda_stream))
@@ -298,6 +358,31 @@ class MonoBatch:
             a = native.stereo_offset
             inputs["stereo_T"] = flat[a:a + B * _STEREO_BYTES].view(torch.float32).view(B, 4, 4)
         return inputs
+
+    def _decode_jpeg(self, native: NativeBatch, flat: torch.Tensor) -> torch.Tensor:
+        """The device native-frame buffer of a batch with JPEG frames: decoded, and the host-decoded frames copied."""
+        cap = self.jpeg_capacity or (native.native_bytes, native.jpeg_chunks * jpeg.CHUNK_BYTES, native.jpeg_blocks)
+        need = (native.native_bytes, native.jpeg_chunks * jpeg.CHUNK_BYTES, native.jpeg_blocks)
+        if any(n > c for n, c in zip(need, cap)):
+            raise ValueError("batch needs (native bytes, entropy bytes, blocks) = %s, over MonoBatch's jpeg_capacity %s"
+                             % (need, cap))
+        n = len(native.jpeg_names)
+        frames = torch.empty(cap[0], dtype=torch.uint8, device=flat.device)
+        for src, dst, nbytes in native.jpeg_copies:        # host-decoded frames: one cudaMemcpyAsync each
+            frames[dst:dst + nbytes].copy_(flat[src:src + nbytes], non_blocking=True)
+        status = torch.empty(n, dtype=torch.int32, device=flat.device)
+        jpeg.run(self.lib, flat, native.buffer.data_ptr() + native.jpeg_jobs_offset, native.jpeg_jobs_offset, n, frames,
+                 status, max(1, cap[1] // jpeg.CHUNK_BYTES), max(1, cap[2]))
+        self.jpeg_status, self._jpeg_names = status, list(native.jpeg_names)
+        return frames
+
+    def check_jpeg(self) -> None:
+        """Synchronises and raises ValueError naming every JPEG file of the last build whose data was corrupt."""
+        if self.jpeg_status is None:
+            return
+        err = jpeg.status_error(self.jpeg_status.cpu().tolist(), self._jpeg_names)
+        if err:
+            raise ValueError(err)
 
     def __call__(self, native: NativeBatch) -> Dict:
         return self.build(native, self.upload(native))
