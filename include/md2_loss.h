@@ -433,6 +433,50 @@ int md2_jpeg_decode(const unsigned char *data, size_t data_bytes, const md2_jpeg
                     int n_images, unsigned char *frames, size_t frames_bytes, unsigned int *status,
                     long long max_chunks, long long max_blocks, void *scratch, size_t scratch_bytes, void *stream);
 
+/* ---- PNG decoding on the GPU: the frames of kitti_dataset.py get_color for KITTI's own .png files, pil_loader's
+ * Image.open(f).convert("RGB"), byte for byte what Pillow gives, for 8-bit truecolour non-interlaced PNGs.
+ *
+ * The host (monodepth2_b200/png.py) checks the chunks and the 2-byte zlib header and lays out per image, inside
+ * `data`, the concatenated IDAT payloads from the first byte after the zlib header: the deflate data, and after it
+ * whatever the file holds (the Adler-32 trailer, or nothing, or more).  Images are numbered across the call by two
+ * running sums: stream_index over stream_bytes and raw_offset over the inflated size height * (3 * width + 1).  The
+ * image is written as (height, width, 3) uint8 HWC at byte out_offset of `frames`.
+ *
+ * The Adler-32 trailer is read where zlib reads it, from the byte after the final block, and checked when all four
+ * bytes are present and the inflated data is complete there or shorter (zlib's stream end).  A stream that ends a
+ * positive whole number of rows short with a good trailer gives the image with zero rows after it, as Pillow does;
+ * any other early end is MD2_PNG_EXHAUSTED.  One case differs from Pillow: Pillow feeds zlib one IDAT piece (at most
+ * 64 KB) at a time and skips the check of a complete image's trailer when the trailer is not in the piece that
+ * completes the last row; here it is always checked.  status (device, n_images
+ * uint32) gets per image the MD2_PNG_* bits below; 0 is a clean decode.  A stream that sets one may leave any bytes
+ * in its frame, but the call never reads or writes outside its buffers.  The scratch size depends only on n_images
+ * and the capacity (max_stream_bytes, max_raw_bytes); md2_png_decode only enqueues (a memset and six kernels), so
+ * one allocation and one captured CUDA graph serve every batch within the capacity.  `jobs` is read on the host for
+ * validation, `jobs_dev` (the same records on the device) by the kernels. ---- */
+#define MD2_PNG_BAD_CODE 1u           /* an invalid block type, code set, code, repeat or stored length */
+#define MD2_PNG_DISTANCE 2u           /* a distance back past the start of the data */
+#define MD2_PNG_EXHAUSTED 4u          /* the data ended before the last row (truncated, or too little output) */
+#define MD2_PNG_BAD_FILTER 8u         /* a row's filter type above 4 */
+#define MD2_PNG_CHECKSUM 16u          /* the Adler-32 trailer differs from the inflated data's */
+#define MD2_PNG_CAPACITY 32u          /* the image lies outside the buffers or the capacity (a replayed CUDA graph
+                                         fed a larger batch): skipped */
+#define MD2_PNG_MAX_SIDE 16384
+typedef struct md2_png_job {
+  long long out_offset;               /* byte offset of the decoded frame in `frames` */
+  long long stream_offset;            /* byte offset of the stream in `data`, 4-byte aligned; data holds it rounded up
+                                         to whole 4-byte words */
+  long long stream_index;             /* running sum of stream_bytes over the images before */
+  long long raw_offset;               /* running sum of height * (3 * width + 1) over the images before */
+  int stream_bytes;
+  int height, width;                  /* 1..MD2_PNG_MAX_SIDE */
+  int reserved;
+} md2_png_job;
+int md2_png_decode_scratch_bytes(int n_images, long long max_stream_bytes, long long max_raw_bytes, size_t *bytes);
+int md2_png_decode(const unsigned char *data, size_t data_bytes, const md2_png_job *jobs, const md2_png_job *jobs_dev,
+                   int n_images, unsigned char *frames, size_t frames_bytes, unsigned int *status,
+                   long long max_stream_bytes, long long max_raw_bytes, void *scratch, size_t scratch_bytes,
+                   void *stream);
+
 #ifdef __cplusplus
 }
 #endif

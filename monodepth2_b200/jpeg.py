@@ -5,7 +5,7 @@ dataloader worker only walks the file's markers (``parse_jpeg``: derived Huffman
 entropy-coded segments with stuffing and restart markers removed), ``collate_native`` packs the compressed streams,
 and ``MonoBatch`` decodes them on the device into the native-frame buffer its batch builder reads.  A file outside the
 supported class (progressive, arithmetic-coded, 12-bit, grayscale, CMYK or RGB, other samplings, PNG) is decoded on
-the host by the dataset's own ``get_color``, as before.
+the host by the dataset's own ``get_color``, as before (PNG files on the device, with ``png.PngFramesMixin`` in front).
 
     class GpuKITTIRAW(JpegFramesMixin, NativeFramesMixin, KITTIRAWDataset): pass
     loader = DataLoader(GpuKITTIRAW(...), ..., collate_fn=collate_native)

@@ -23,7 +23,7 @@ from typing import Dict, List, Optional
 import numpy as np
 import torch
 
-from . import _capi, jpeg, kitti_depth
+from . import _capi, jpeg, kitti_depth, png
 from .pyramid import ColorAug
 
 # KITTIDataset.K (kitti_dataset.py): intrinsics normalised by the image size
@@ -38,6 +38,7 @@ JOB_DTYPE = np.dtype([("offset", "<i8"), ("height", "<i4"), ("width", "<i4"), ("
 _PARAM_BYTES = 32           # one md2_color_jitter row
 _STEREO_BYTES = 64          # one 4x4 float32 stereo_T
 _DRAW_KEYS = ("frames", "do_color_aug", "do_flip", "color_aug", "side", "velodyne")
+_COMPRESSED = (jpeg.JpegStream, png.PngStream)
 
 
 def _align(n: int, a: int = 16) -> int:
@@ -69,16 +70,24 @@ class NativeBatch:
     velo_jobs_offset: int = -1  # -1 without velodyne scans
     velo_out_shape: Optional[tuple] = None
     # Items from JpegFramesMixin: the md2_jpeg_job table of the JPEG frames at jpeg_jobs_offset (after the scans' job
-    # table, so its place depends only on the batch size and the frame ids), their compressed streams after the
-    # frames and scans.  The job table's frame offsets then index a device native-frame buffer of native_bytes, into
-    # which the JPEG frames are decoded and the host-decoded frames (jpeg_copies: (offset in buffer, offset in that
-    # device buffer, bytes)) are copied.
+    # table, and after the PNG frames' when there are any, so without PNG frames its place depends only on the batch
+    # size and the frame ids), their compressed streams after the frames and scans.  The job table's frame offsets
+    # then index a device native-frame buffer of native_bytes, into which the JPEG (and PNG) frames are decoded and
+    # the host-decoded frames (jpeg_copies: (offset in buffer, offset in that device buffer, bytes)) are copied.
     jpeg_jobs_offset: int = -1
     jpeg_names: Optional[list] = None
     jpeg_chunks: int = 0
     jpeg_blocks: int = 0
     native_bytes: int = 0
     jpeg_copies: Optional[list] = None
+    # Items from PngFramesMixin: the md2_png_job table of the PNG frames at png_jobs_offset (right after the scans' job
+    # table: its place depends only on the batch size and the frame ids), their deflate streams after the JPEG
+    # streams; png_stream_bytes / png_raw_bytes are the batch's deflate and inflated bytes.  They share the device
+    # native-frame buffer and the copy list above with the JPEG frames.
+    png_jobs_offset: int = -1
+    png_names: Optional[list] = None
+    png_stream_bytes: int = 0
+    png_raw_bytes: int = 0
 
     @property
     def n_images(self) -> int:
@@ -106,10 +115,11 @@ def collate_native(items: List[dict], pin_memory: Optional[bool] = None) -> Nati
             raise ValueError("every item of a batch must hold the same frame ids")
     n = B * len(fids)
     frames = [items[b]["frames"][f] for f in fids for b in range(B)]
-    frames = [a if isinstance(a, jpeg.JpegStream) else np.ascontiguousarray(a, dtype=np.uint8) for a in frames]
+    frames = [a if isinstance(a, _COMPRESSED) else np.ascontiguousarray(a, dtype=np.uint8) for a in frames]
     streams = [a for a in frames if isinstance(a, jpeg.JpegStream)]
+    pngs = [a for a in frames if isinstance(a, png.PngStream)]
     for a in frames:
-        if isinstance(a, jpeg.JpegStream):
+        if isinstance(a, _COMPRESSED):
             continue
         if a.ndim != 3 or a.shape[2] != 3:
             raise ValueError("native frames must be (h, w, 3) uint8 arrays, got %s" % (a.shape,))
@@ -126,6 +136,10 @@ def collate_native(items: List[dict], pin_memory: Optional[bool] = None) -> Nati
             raise ValueError("every velodyne scan of a batch must give the same depth_gt size")
         velo_off = off
         off = _align(off + B * kitti_depth.VELO_JOB_DTYPE.itemsize)
+    png_off = -1
+    if pngs:
+        png_off = off
+        off = _align(off + len(pngs) * png.JOB_DTYPE.itemsize, 64)
     jpeg_off = -1
     if streams:
         jpeg_off = off
@@ -137,10 +151,10 @@ def collate_native(items: List[dict], pin_memory: Optional[bool] = None) -> Nati
         total = _align(total + a.nbytes)
     native_total = total
     copies = None
-    if streams:                 # the buffer holds only the host-decoded frames; rel indexes the device frame buffer
+    if streams or pngs:         # the buffer holds only the host-decoded frames; rel indexes the device frame buffer
         copies, total = [], 0
         for a, r in zip(frames, rel):
-            if not isinstance(a, jpeg.JpegStream):
+            if not isinstance(a, _COMPRESSED):
                 copies.append((frames_off + total, r, a.nbytes))
                 total = _align(total + a.nbytes)
     if velo is not None:        # the scans after the frames; their job records hold their offsets
@@ -149,6 +163,9 @@ def collate_native(items: List[dict], pin_memory: Optional[bool] = None) -> Nati
     if streams:
         body_off = _align(frames_off + total, 64)
         total = body_off - frames_off + jpeg.body_bytes(streams)
+    if pngs:
+        png_body_off = _align(frames_off + total, 64)
+        total = png_body_off - frames_off + png.body_bytes(pngs)
     if pin_memory is None:
         pin_memory = get_worker_info() is None and torch.cuda.is_available()
     buf = torch.empty(frames_off + total, dtype=torch.uint8, pin_memory=bool(pin_memory))
@@ -174,7 +191,7 @@ def collate_native(items: List[dict], pin_memory: Optional[bool] = None) -> Nati
         for a, r in zip(frames, rel):
             h[frames_off + r:frames_off + r + a.nbytes] = a.reshape(-1)
     else:
-        for a, (src, _, nb) in zip([a for a in frames if not isinstance(a, jpeg.JpegStream)], copies):
+        for a, (src, _, nb) in zip([a for a in frames if not isinstance(a, _COMPRESSED)], copies):
             h[src:src + nb] = a.reshape(-1)
     if velo is not None:
         kitti_depth.pack_jobs(h, velo_off, scans_off, velo, do_flip, False)
@@ -182,12 +199,17 @@ def collate_native(items: List[dict], pin_memory: Optional[bool] = None) -> Nati
     if streams:
         chunks, blocks = jpeg.pack(h, jpeg_off, body_off, streams,
                                    [r for a, r in zip(frames, rel) if isinstance(a, jpeg.JpegStream)])
+    png_stream = png_raw = 0
+    if pngs:
+        png_stream, png_raw = png.pack(h, png_off, png_body_off, pngs,
+                                       [r for a, r in zip(frames, rel) if isinstance(a, png.PngStream)])
     extra_keys = [k for k in items[0] if k not in _DRAW_KEYS]
     extra = default_collate([{k: it[k] for k in extra_keys} for it in items]) if extra_keys else {}
     return NativeBatch(buf, B, fids, 0, stereo_off, jobs_off, frames_off,
                        torch.tensor([bool(it["do_color_aug"]) for it in items]), torch.tensor(do_flip), draws, sides, extra,
                        velo_off, tuple(velo[0].out_shape) if velo is not None else None, jpeg_off,
-                       [s.name for s in streams], chunks, blocks, native_total, copies)
+                       [s.name for s in streams], chunks, blocks, native_total, copies, png_off,
+                       [s.name for s in pngs], png_stream, png_raw)
 
 
 class NativeFramesMixin:
@@ -225,7 +247,7 @@ class NativeFramesMixin:
 
     def native_color(self, folder, frame_index, side):
         """A native frame: the dataset's ``get_color(folder, frame_index, side, False)`` as an (h, w, 3) uint8 array
-        (``JpegFramesMixin`` returns the parsed JPEG instead)."""
+        (``JpegFramesMixin`` and ``PngFramesMixin`` return the parsed file instead)."""
         return np.array(self.get_color(folder, frame_index, side, False))
 
     def native_depth(self, folder, frame_index, side, do_flip) -> dict:
@@ -251,10 +273,16 @@ class MonoBatch:
     out); a batch over it raises before anything is enqueued.  With a capacity, a graph captured on one batch replays
     batches of other compressed lengths and native sizes that hold as many JPEG frames and no host-decoded frame;
     without, each batch is sized to itself.  ``jpeg_status`` is the device status word of every JPEG frame of the last
-    build (read without synchronising); ``check_jpeg()`` synchronises and raises naming the corrupt files."""
+    build (read without synchronising); ``check_jpeg()`` synchronises and raises naming the corrupt files.
+
+    Batches of ``PngFramesMixin`` items are decoded the same way (``md2_png_decode``) into the same buffer, next to
+    any JPEG and host-decoded frames.  ``png_capacity = (native_bytes, stream_bytes, raw_bytes)`` sizes it as
+    ``jpeg_capacity`` does (``stream_bytes``: the frames' deflate data, ``raw_bytes``: their inflated size,
+    ``height * (3 * width + 1)`` each); the buffer takes the larger native_bytes of the two.  ``png_status`` and
+    ``check_png()`` report the PNG frames as their JPEG counterparts do."""
 
     def __init__(self, height: int, width: int, frame_ids, num_scales: int = 4, K=None,
-                 color_dtype: torch.dtype = torch.uint8, device=None, jpeg_capacity=None):
+                 color_dtype: torch.dtype = torch.uint8, device=None, jpeg_capacity=None, png_capacity=None):
         if color_dtype not in (torch.uint8, torch.float32):
             raise ValueError("color_dtype must be torch.uint8 or torch.float32")
         self.height, self.width, self.num_scales = int(height), int(width), int(num_scales)
@@ -278,6 +306,9 @@ class MonoBatch:
         self.jpeg_capacity = None if jpeg_capacity is None else tuple(int(v) for v in jpeg_capacity)
         self.jpeg_status: Optional[torch.Tensor] = None
         self._jpeg_names: list = []
+        self.png_capacity = None if png_capacity is None else tuple(int(v) for v in png_capacity)
+        self.png_status: Optional[torch.Tensor] = None
+        self._png_names: list = []
 
     def __del__(self):
         try:
@@ -329,8 +360,8 @@ class MonoBatch:
         scratch = torch.empty(nb.value, dtype=torch.uint8, device=dev)
         base = flat.data_ptr()
         frames_ptr, frames_bytes = base + native.frames_offset, flat.numel() - native.frames_offset
-        if native.jpeg_jobs_offset >= 0:
-            frames = self._decode_jpeg(native, flat)
+        if native.jpeg_jobs_offset >= 0 or native.png_jobs_offset >= 0:
+            frames = self._native_frames(native, flat)
             frames_ptr, frames_bytes = frames.data_ptr(), frames.numel()
         with torch.cuda.device(dev):
             st = self.lib.md2_batch_build_u8(
@@ -359,21 +390,41 @@ class MonoBatch:
             inputs["stereo_T"] = flat[a:a + B * _STEREO_BYTES].view(torch.float32).view(B, 4, 4)
         return inputs
 
-    def _decode_jpeg(self, native: NativeBatch, flat: torch.Tensor) -> torch.Tensor:
-        """The device native-frame buffer of a batch with JPEG frames: decoded, and the host-decoded frames copied."""
-        cap = self.jpeg_capacity or (native.native_bytes, native.jpeg_chunks * jpeg.CHUNK_BYTES, native.jpeg_blocks)
-        need = (native.native_bytes, native.jpeg_chunks * jpeg.CHUNK_BYTES, native.jpeg_blocks)
-        if any(n > c for n, c in zip(need, cap)):
-            raise ValueError("batch needs (native bytes, entropy bytes, blocks) = %s, over MonoBatch's jpeg_capacity %s"
-                             % (need, cap))
-        n = len(native.jpeg_names)
-        frames = torch.empty(cap[0], dtype=torch.uint8, device=flat.device)
+    def _native_frames(self, native: NativeBatch, flat: torch.Tensor) -> torch.Tensor:
+        """The device native-frame buffer of a batch with compressed frames: the host-decoded frames copied, the JPEG
+        and PNG frames decoded."""
+        jobs = []                   # (decoder, capacity, need); a capacity's first entry sizes the native-frame buffer
+        if native.jpeg_jobs_offset >= 0:
+            need = (native.native_bytes, native.jpeg_chunks * jpeg.CHUNK_BYTES, native.jpeg_blocks)
+            cap = self.jpeg_capacity or need
+            if any(n > c for n, c in zip(need, cap)):
+                raise ValueError("batch needs (native bytes, entropy bytes, blocks) = %s, over MonoBatch's "
+                                 "jpeg_capacity %s" % (need, cap))
+            jobs.append(("jpeg", cap))
+        if native.png_jobs_offset >= 0:
+            need = (native.native_bytes, native.png_stream_bytes, native.png_raw_bytes)
+            cap = self.png_capacity or need
+            if any(n > c for n, c in zip(need, cap)):
+                raise ValueError("batch needs (native bytes, stream bytes, raw bytes) = %s, over MonoBatch's "
+                                 "png_capacity %s" % (need, cap))
+            jobs.append(("png", cap))
+        frames = torch.empty(max(cap[0] for _, cap in jobs), dtype=torch.uint8, device=flat.device)
         for src, dst, nbytes in native.jpeg_copies:        # host-decoded frames: one cudaMemcpyAsync each
             frames[dst:dst + nbytes].copy_(flat[src:src + nbytes], non_blocking=True)
-        status = torch.empty(n, dtype=torch.int32, device=flat.device)
-        jpeg.run(self.lib, flat, native.buffer.data_ptr() + native.jpeg_jobs_offset, native.jpeg_jobs_offset, n, frames,
-                 status, max(1, cap[1] // jpeg.CHUNK_BYTES), max(1, cap[2]))
-        self.jpeg_status, self._jpeg_names = status, list(native.jpeg_names)
+        host = native.buffer.data_ptr()
+        for kind, cap in jobs:
+            if kind == "jpeg":
+                n = len(native.jpeg_names)
+                status = torch.empty(n, dtype=torch.int32, device=flat.device)
+                jpeg.run(self.lib, flat, host + native.jpeg_jobs_offset, native.jpeg_jobs_offset, n, frames, status,
+                         max(1, cap[1] // jpeg.CHUNK_BYTES), max(1, cap[2]))
+                self.jpeg_status, self._jpeg_names = status, list(native.jpeg_names)
+            else:
+                n = len(native.png_names)
+                status = torch.empty(n, dtype=torch.int32, device=flat.device)
+                png.run(self.lib, flat, host + native.png_jobs_offset, native.png_jobs_offset, n, frames, status,
+                        max(1, cap[1]), max(1, cap[2]))
+                self.png_status, self._png_names = status, list(native.png_names)
         return frames
 
     def check_jpeg(self) -> None:
@@ -381,6 +432,14 @@ class MonoBatch:
         if self.jpeg_status is None:
             return
         err = jpeg.status_error(self.jpeg_status.cpu().tolist(), self._jpeg_names)
+        if err:
+            raise ValueError(err)
+
+    def check_png(self) -> None:
+        """Synchronises and raises ValueError naming every PNG file of the last build whose data was corrupt."""
+        if self.png_status is None:
+            return
+        err = png.status_error(self.png_status.cpu().tolist(), self._png_names)
         if err:
             raise ValueError(err)
 
